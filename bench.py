@@ -1,6 +1,7 @@
 """bench.py — ADMM iterations/s of the full-vertex-split iteration (reference admm_solver_v3.py:655-733) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload grid316|grid100|grid1000|batch4096] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one ADMM iteration (K1 vertex programs + the fused edge / dual / residual / control kernel) over the whole
 workload.  `value` = iterations/s with everything resident in HBM (CUDA events on the library's stream, L2 flushed before
@@ -89,6 +90,26 @@ def build_workload(name, rank=0, world=1):
         return g, (f"batch of {nq} independent benchmark4-sized start/goal queries (s, t in one component of the region graph), "
                    f"{len(qs)} on this GPU: {g.nV} vertices, {g.nE} directed edges, block-diagonal, per-problem residuals / rho / stop")
     raise SystemExit(f"unknown workload {name!r}")
+
+
+DUMP_BYTES = 60 * 10 ** 6        # payload cap of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes every array of `outputs` (one row per vertex, edge or problem) as <out_dir>/<name>.npy in float64.  When
+    together they exceed DUMP_BYTES (the million-vertex grid, long runs of a batch), each keeps the same fraction of its
+    rows, at least one, drawn by default_rng(0) and kept in order: the sample depends only on the array's length, so two
+    runs with the same arguments store the same rows."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in outputs.items()}
+    one_row = sum(a[:1].nbytes for a in arrays.values())
+    if one_row > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: one row of every output is {one_row} bytes, more than the {DUMP_BYTES} allowed; use fewer --steps")
+    frac = min(1.0, (DUMP_BYTES - one_row) / sum(a.nbytes for a in arrays.values()))    # sum of max(1, n * frac) rows <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        if frac < 1.0:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], max(1, int(a.shape[0] * frac)), replace=False))]
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def steady_state(g, burn, mode="parity", tables=None, inner=1):
@@ -224,13 +245,18 @@ def main():
                     help="seconds allowed for the time-to-residual-1e-4 run (perf mode); -1: 330 for the metric workload on 1 GPU, else 0; N > 1: any value > 0 enables the run (bounded by --residual-cap)")
     ap.add_argument("--residual-cap", type=int, default=1_200_000, help="N > 1: iteration cap of the time-to-residual run (ranks cannot agree on a wall-clock budget)")
     ap.add_argument("--outer-alpha", type=float, default=1.0, help="over-relaxation of the consensus step in the time-to-residual run")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="1 GPU: write what the timed path returns after its last step (solution x_v, z_v, y_v, z_e; rho / pri_res / dual_res "
+                         "of the timed steps, one row per problem of a batch) as DIR/<name>.npy, float64, at most 64 MB (a seeded row sample of larger outputs)")
     args = ap.parse_args()
     if args.grid:
         WORKLOADS.setdefault(f"grid{args.grid}", args.grid)
         args.workload = f"grid{args.grid}"
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl == "reference" or world > 1 or args.gpus > 1):
+        ap.error("--dump-outputs is implemented for the single-GPU path only")
     if args.impl == "reference":
         return run_reference(args)
-    world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1 or args.gpus > 1:
         from gcs_admm_b200 import dist_bench  # multi-GPU path (vertex-partitioned grids / sharded query batches)
         import gcs_admm_b200  # noqa: F401
@@ -251,8 +277,9 @@ def main():
     if args.mode == "perf" and gate and not gate["passed"]:
         headline = "parity"        # the gate decides, not the flag
 
-    def timed(mode, steps, burn_it):
-        """burn-in, then `steps` iterations timed one by one with CUDA events on the solver's stream, L2 flushed before each"""
+    def timed(mode, steps, burn_it, keep_outputs=False):
+        """burn-in, then `steps` iterations timed one by one with CUDA events on the solver's stream, L2 flushed before each;
+        keep_outputs: also return what a caller of this path receives after the last timed iteration"""
         s = lib.Solver(g, device=0, max_it=max(1000, steps + burn_it + 8), eps_abs=0.0, eps_rel=0.0)
         if mode == "perf":
             s.enable_perf(inner_iters=args.inner, tables=tables)
@@ -268,8 +295,20 @@ def main():
         clocks = sampler.finish()
         st = s.status()
         state = list(s.state()) + (list(s.perf_state()) if mode == "perf" else [])
+        outputs = None
+        if keep_outputs:
+            outputs = dict(zip(("x_v", "z_v", "y_v", "z_e"), s.solution()))
+            # rho / residuals of the timed iterations, one row per problem (a batch keeps them per problem); NaN after a
+            # problem's own stop
+            n_prob = len(g.prob_voff) - 1 if getattr(g, "prob_voff", None) is not None else 1
+            hist = np.full((3, n_prob, steps), np.nan)
+            for p in range(n_prob):
+                for q, h in enumerate(s.problem_history(p)):
+                    seg = h[st0["iterations"] + 1: st0["iterations"] + 1 + steps]
+                    hist[q, p, :len(seg)] = seg
+            outputs.update(zip(("rho", "pri_res", "dual_res"), hist))
         s.close()
-        return dict(ms=tot / steps, k1_ms=k1 / steps, ed_ms=ed / steps, clocks=clocks, st0=st0, st=st, state=state)
+        return dict(ms=tot / steps, k1_ms=k1 / steps, ed_ms=ed / steps, clocks=clocks, st0=st0, st=st, state=state, outputs=outputs)
 
     def end_to_end(mode, state, n):
         """host buffers -> host buffers through the C-ABI, wall clock: graph / tables / warm state upload + n iterations + download"""
@@ -295,7 +334,9 @@ def main():
             gs += sum(np.asarray(tables[k]).nbytes for k in ("vclass", "cls_tab", "cone_off", "cone", "blk_off", "blk_he", "blk_info", "tile_voff"))
         return gs
 
-    m = timed(headline, args.steps, burn)
+    m = timed(headline, args.steps, burn, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, m["outputs"])
     ms, k1_ms, ed_ms, clocks = m["ms"], m["k1_ms"], m["ed_ms"], m["clocks"]
     e2e_s = end_to_end(headline, m["state"], args.steps)
     n_long = 1000 if headline == "perf" else 50

@@ -46,25 +46,14 @@ def test_problem_files_load_and_match_fixtures(name):
         assert np.array_equal(As[k], Ag[k]) and np.array_equal(bs[k], bg[k])
 
 
-def test_reference_problem_files_load_unmodified():
-    ref = "/root/reference/test_data"
-    if not os.path.isdir(ref):
-        pytest.skip("reference checkout not present (GPU box)")
-    from gcs_admm_b200.problem_io import load_test_file
-    for name in ALL_PROBLEMS:
-        As, bs, n = load_test_file(name, ref)
-        Ag, bg, ng, d, keys = load_golden(name)
-        assert list(As.keys()) == keys and all(np.array_equal(As[k], Ag[k]) for k in keys)
-    with pytest.raises(ModuleNotFoundError):
-        load_test_file("does_not_exist", ref)
-
-
 def test_write_then_load_roundtrip(tmp_path):
     from gcs_admm_b200.problem_io import load_test_file, write_test_file
     As, bs, n, d, keys = load_golden("benchmark2")
     write_test_file(str(tmp_path / "rt.py"), As, bs, s=d["s"], t=d["t"])
     A2, b2, n2 = load_test_file("rt", str(tmp_path))
     assert list(A2.keys()) == keys and all(np.array_equal(A2[k], As[k]) and np.array_equal(b2[k], bs[k]) for k in keys)
+    with pytest.raises(ModuleNotFoundError):
+        load_test_file("does_not_exist", str(tmp_path))
 
 
 @pytest.mark.parametrize("name", ["benchmark1", "benchmark2", "benchmark3", "benchmark4"])
