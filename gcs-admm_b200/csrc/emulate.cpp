@@ -33,15 +33,18 @@ extern "C" int gcsemu_vertex_update_all(int nV, int nE, const int *poly_off, con
 extern "C" int gcsemu_scratch_doubles(int dcap, int mcap) { return gcs_scratch_layout(dcap, mcap).total; }
 extern "C" int gcsemu_ws_stride(int dcap, int mcap) { return gcs_ws_stride(gcs_scratch_layout(dcap, mcap)); }
 
-// perf-mode K1 (vertex_perf.cuh), emulated: one host thread plays each thread block (tile) in turn
-extern "C" int gcsemu_vertex_update_perf_all(int nV, int nE, const int *poly_off, const double *polyA, const double *polyb,
-                                             const int *he_off, const int *he_edge, const unsigned char *he_flags,
-                                             const unsigned char *vtype, const double *cent, double *xc, const double *mu,
-                                             const double *z, double *x_v, double *z_v, double *y_v, double rho, double mu_scale,
-                                             const int *vclass, const double *cls_tab, const int *cone_off, const double *cone,
-                                             const int *blk_off, const int *blk_he, const int *blk_edge, const int *blk_info, const int *tile_voff, int ntiles,
-                                             int cap_blocks, int cap_verts, int cap_cone, double *tstate, double *tn,
-                                             int inner_iters, double alpha, double kappa, double theta, const double *edge_delta) {
+// perf-mode K1 (vertex_perf.cuh), emulated: one host thread plays each thread block (tile) in turn.
+// INNER: the variant that also measures the inner residual; each tile's share goes to rin_tile[t] (summed by the caller in
+// tile order, so the result does not depend on the OpenMP schedule)
+template <bool INNER>
+static int perf_all(int nV, int nE, const int *poly_off, const double *polyA, const double *polyb,
+                    const int *he_off, const int *he_edge, const unsigned char *he_flags,
+                    const unsigned char *vtype, const double *cent, double *xc, const double *mu,
+                    const double *z, double *x_v, double *z_v, double *y_v, double rho, double mu_scale,
+                    const int *vclass, const double *cls_tab, const int *cone_off, const double *cone,
+                    const int *blk_off, const int *blk_he, const int *blk_edge, const int *blk_info, const int *tile_voff, int ntiles,
+                    int cap_blocks, int cap_verts, int cap_cone, double *tstate, double *tn,
+                    int inner_iters, double alpha, double kappa, double theta, const double *edge_delta, double *rin_tile) {
     GcsGraphView G = {nV, nE, poly_off, polyA, polyb, he_off, he_edge, he_flags, vtype, cent};
     GcsStateView St = {xc, mu, z, x_v, z_v, y_v, 0, 0.0, 0.0};
     GcsPerfLayout L = gcs_perf_layout(cap_blocks, cap_verts, cap_cone);
@@ -75,7 +78,8 @@ extern "C" int gcsemu_vertex_update_perf_all(int nV, int nE, const int *poly_off
             memset(S, poison, sizeof(double) * L.total);
             Ctrl local = ctrl;
             double rin = 0.0;
-            gcs_perf_tile<false>(G, St, T, L, S, S + L.work, t, &local, 0, rin);
+            gcs_perf_tile<INNER>(G, St, T, L, S, S + L.work, t, &local, 0, rin);
+            if (rin_tile) rin_tile[t] = rin;
         }
         free(S);
     }
@@ -83,4 +87,43 @@ extern "C" int gcsemu_vertex_update_perf_all(int nV, int nE, const int *poly_off
     for (int v = 0; v < nV; ++v)      // what perf_init_dead_kernel writes once on the device
         if (vtype[v] == GCS_VT_DEAD) { for (int k = 0; k < 4; ++k) { z_v[4 * v + k] = 0.0; x_v[4 * v + k] = cent[2 * v + (k & 1)]; } y_v[v] = 0.0; }
     return ntiles;
+}
+
+extern "C" int gcsemu_vertex_update_perf_all(int nV, int nE, const int *poly_off, const double *polyA, const double *polyb,
+                                             const int *he_off, const int *he_edge, const unsigned char *he_flags,
+                                             const unsigned char *vtype, const double *cent, double *xc, const double *mu,
+                                             const double *z, double *x_v, double *z_v, double *y_v, double rho, double mu_scale,
+                                             const int *vclass, const double *cls_tab, const int *cone_off, const double *cone,
+                                             const int *blk_off, const int *blk_he, const int *blk_edge, const int *blk_info, const int *tile_voff, int ntiles,
+                                             int cap_blocks, int cap_verts, int cap_cone, double *tstate, double *tn,
+                                             int inner_iters, double alpha, double kappa, double theta, const double *edge_delta) {
+    return perf_all<false>(nV, nE, poly_off, polyA, polyb, he_off, he_edge, he_flags, vtype, cent, xc, mu, z, x_v, z_v, y_v, rho, mu_scale,
+                           vclass, cls_tab, cone_off, cone, blk_off, blk_he, blk_edge, blk_info, tile_voff, ntiles, cap_blocks, cap_verts,
+                           cap_cone, tstate, tn, inner_iters, alpha, kappa, theta, edge_delta, nullptr);
+}
+
+// the INNER variant of K1 (what the device runs once the run is near its absolute tolerance): the same update, plus
+// *inner_sq = the squared inner residual |(M u + m0) - c|^2 over every pair and path-length item of the last pass
+extern "C" int gcsemu_vertex_update_perf_inner(int nV, int nE, const int *poly_off, const double *polyA, const double *polyb,
+                                               const int *he_off, const int *he_edge, const unsigned char *he_flags,
+                                               const unsigned char *vtype, const double *cent, double *xc, const double *mu,
+                                               const double *z, double *x_v, double *z_v, double *y_v, double rho, double mu_scale,
+                                               const int *vclass, const double *cls_tab, const int *cone_off, const double *cone,
+                                               const int *blk_off, const int *blk_he, const int *blk_edge, const int *blk_info, const int *tile_voff, int ntiles,
+                                               int cap_blocks, int cap_verts, int cap_cone, double *tstate, double *tn,
+                                               int inner_iters, double alpha, double kappa, double theta, const double *edge_delta, double *inner_sq) {
+    double *rin = (double *)calloc((size_t)(ntiles > 0 ? ntiles : 1), sizeof(double));
+    const int r = perf_all<true>(nV, nE, poly_off, polyA, polyb, he_off, he_edge, he_flags, vtype, cent, xc, mu, z, x_v, z_v, y_v, rho, mu_scale,
+                                 vclass, cls_tab, cone_off, cone, blk_off, blk_he, blk_edge, blk_info, tile_voff, ntiles, cap_blocks, cap_verts,
+                                 cap_cone, tstate, tn, inner_iters, alpha, kappa, theta, edge_delta, rin);
+    double s = 0.0;
+    for (int t = 0; t < ntiles; ++t) s += rin[t];       // tile order: independent of the OpenMP schedule
+    *inner_sq = s;
+    free(rin);
+    return r;
+}
+
+// gcs_cone_project on n points (pts, out: n x 3) against one cone of nv records (GCS_CONE_REC doubles each)
+extern "C" void gcsemu_cone_project(const double *cone, int nv, const double *pts, int n, double *out) {
+    for (int i = 0; i < n; ++i) gcs_cone_project(cone, nv, pts[3 * i], pts[3 * i + 1], pts[3 * i + 2], out[3 * i], out[3 * i + 1], out[3 * i + 2]);
 }

@@ -24,10 +24,15 @@ _bp = np.ctypeslib.ndpointer(dtype=np.uint8, flags="C_CONTIGUOUS")
 def load_emu():
     from conftest import build_emu
     lib = C.CDLL(build_emu())
+    perf_args = [C.c_int, C.c_int, _ip, _dp, _dp, _ip, _ip, _bp, _bp, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
+                 C.c_double, C.c_double, _ip, _dp, _ip, _dp, _ip, _ip, _ip, _ip, _ip, C.c_int,
+                 C.c_int, C.c_int, C.c_int, _dp, _dp, C.c_int, C.c_double, C.c_double, C.c_double, C.c_void_p]
     lib.gcsemu_vertex_update_perf_all.restype = C.c_int
-    lib.gcsemu_vertex_update_perf_all.argtypes = [C.c_int, C.c_int, _ip, _dp, _dp, _ip, _ip, _bp, _bp, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
-                                                  C.c_double, C.c_double, _ip, _dp, _ip, _dp, _ip, _ip, _ip, _ip, _ip, C.c_int,
-                                                  C.c_int, C.c_int, C.c_int, _dp, _dp, C.c_int, C.c_double, C.c_double, C.c_double, C.c_void_p]
+    lib.gcsemu_vertex_update_perf_all.argtypes = perf_args
+    lib.gcsemu_vertex_update_perf_inner.restype = C.c_int
+    lib.gcsemu_vertex_update_perf_inner.argtypes = perf_args + [C.POINTER(C.c_double)]
+    lib.gcsemu_cone_project.restype = None
+    lib.gcsemu_cone_project.argtypes = [_dp, C.c_int, _dp, C.c_int, _dp]
     return lib
 
 
@@ -49,16 +54,25 @@ class EmuPerfADMM:
         self.x_v, self.z_v, self.y_v = np.zeros((g.nV, 4)), np.zeros((g.nV, 4)), np.zeros(g.nV)
         self.cent = np.ascontiguousarray(g.interior_points())
         self.rho, self.ms, self.pri, self.dual = 1.0, 1.0, [0.0], [0.0]
+        self.inner = False                   # True: vertex_update runs the INNER variant of K1 and sets inner_sq
+        self.inner_sq = None
 
     def vertex_update(self):
+        """inner = True: the INNER variant of K1, which also leaves the squared inner residual of this update in inner_sq"""
         g, T = self.g, self.T
-        self.lib.gcsemu_vertex_update_perf_all(g.nV, g.nE, g.poly_off, g.polyA.reshape(-1), g.polyb, g.he_off, g.he_edge, g.he_flags,
-                                               g.vtype, self.cent.reshape(-1), self.xc.reshape(-1), self.mu.reshape(-1), self.z.reshape(-1),
-                                               self.x_v.reshape(-1), self.z_v.reshape(-1), self.y_v, self.rho, self.ms,
-                                               T["vclass"], T["cls_tab"], T["cone_off"], T["cone"].reshape(-1), T["blk_off"], T["blk_he"],
-                                               self.blk_edge, T["blk_info"], T["tile_voff"], T["tile_voff"].shape[0] - 1, T["caps"]["nb"], T["caps"]["nvt"],
-                                               T["caps"]["cone"], self.tstate.reshape(-1), self.tn.reshape(-1), self.K, self.alpha, T["kappa"], self.theta,
-                                               None if self.delta is None else self.delta.ctypes.data_as(C.c_void_p))
+        args = (g.nV, g.nE, g.poly_off, g.polyA.reshape(-1), g.polyb, g.he_off, g.he_edge, g.he_flags,
+                g.vtype, self.cent.reshape(-1), self.xc.reshape(-1), self.mu.reshape(-1), self.z.reshape(-1),
+                self.x_v.reshape(-1), self.z_v.reshape(-1), self.y_v, self.rho, self.ms,
+                T["vclass"], T["cls_tab"], T["cone_off"], T["cone"].reshape(-1), T["blk_off"], T["blk_he"],
+                self.blk_edge, T["blk_info"], T["tile_voff"], T["tile_voff"].shape[0] - 1, T["caps"]["nb"], T["caps"]["nvt"],
+                T["caps"]["cone"], self.tstate.reshape(-1), self.tn.reshape(-1), self.K, self.alpha, T["kappa"], self.theta,
+                None if self.delta is None else self.delta.ctypes.data_as(C.c_void_p))
+        if self.inner:
+            sq = C.c_double()
+            self.lib.gcsemu_vertex_update_perf_inner(*args, C.byref(sq))
+            self.inner_sq = sq.value
+        else:
+            self.lib.gcsemu_vertex_update_perf_all(*args)
 
     def step_frames(self):
         """local frames: z = argmin |x_head - z|^2 + |x_tail - B z|^2,  B (p1, p2, y) = (p1, p2 - y delta, y)  (gcsadmm.cu edge_frames_kernel)"""
