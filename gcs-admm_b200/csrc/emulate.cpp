@@ -61,7 +61,9 @@ static int perf_all(int nV, int nE, const int *poly_off, const double *polyA, co
         for (int v = a; v < b; ++v) {
             int *w = vrec + GCS_VI_N * v;
             w[GCS_VI_CONE] = cone_off[v] - cone_off[a]; w[GCS_VI_NV] = cone_off[v + 1] - cone_off[v]; w[GCS_VI_CLS] = vclass[v];
-            w[GCS_VI_TERM] = vtype[v] != GCS_VT_GENERIC; w[GCS_VI_BLK] = blk_off[v] - blk_off[a]; w[GCS_VI_NB] = blk_off[v + 1] - blk_off[v];
+            int nin = 0;
+            for (int bb = blk_off[v]; bb < blk_off[v + 1]; ++bb) nin += ((blk_info[bb] >> 8) & 3) == 0;
+            w[GCS_VI_TERM] = (vtype[v] != GCS_VT_GENERIC) | (nin << 1); w[GCS_VI_BLK] = blk_off[v] - blk_off[a]; w[GCS_VI_NB] = blk_off[v + 1] - blk_off[v];
             w[GCS_VI_ACTIVE] = 0; w[GCS_VI_HE] = he_off[v] - he_off[a];
         }
     }
@@ -78,7 +80,7 @@ static int perf_all(int nV, int nE, const int *poly_off, const double *polyA, co
             memset(S, poison, sizeof(double) * L.total);
             Ctrl local = ctrl;
             double rin = 0.0;
-            gcs_perf_tile<INNER>(G, St, T, L, S, S + L.work, t, &local, 0, rin);
+            gcs_perf_tile<INNER, false>(G, St, T, L, S, S + L.work, t, &local, rin, nullptr, 0, nullptr);
             if (rin_tile) rin_tile[t] = rin;
         }
         free(S);
@@ -126,4 +128,12 @@ extern "C" int gcsemu_vertex_update_perf_inner(int nV, int nE, const int *poly_o
 // gcs_cone_project on n points (pts, out: n x 3) against one cone of nv records (GCS_CONE_REC doubles each)
 extern "C" void gcsemu_cone_project(const double *cone, int nv, const double *pts, int n, double *out) {
     for (int i = 0; i < n; ++i) gcs_cone_project(cone, nv, pts[3 * i], pts[3 * i + 1], pts[3 * i + 2], out[3 * i], out[3 * i + 1], out[3 * i + 2]);
+}
+// gcs_cone_project2 on the point pairs (pts[2 i], pts[2 i + 1]), i < n / 2, against one cone (n even; out as for gcsemu_cone_project)
+extern "C" void gcsemu_cone_project2(const double *cone, int nv, const double *pts, int n, double *out) {
+    for (int i = 0; i + 1 < n; i += 2) {
+        const double *c = pts + 3 * i;
+        double *q = out + 3 * i;
+        gcs_cone_project2(cone, nv, c[0], c[1], c[2], c[3], c[4], c[5], q[0], q[1], q[2], q[3], q[4], q[5]);
+    }
 }

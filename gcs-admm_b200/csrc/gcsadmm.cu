@@ -175,12 +175,16 @@ __device__ __forceinline__ void peer_wait_halo(const PeerView &PV) {
 // (<= 256 (point, flow) pairs per tile).  Two stage buffers: while a block computes tile i from one, the bulk copies (TMA unit,
 // mbarrier-signalled) of tile i + gridDim.x fill the other, and the bulk stores of tile i - gridDim.x drain — the DRAM latency of
 // the per-tile state, cone records and descriptors never sits on the critical path.  ~43 KB of shared memory per block.
-template <bool INNER>
+// BATCH: several problems packed block-diagonally (vprob != null); the single-problem variant carries none of their bookkeeping.
+template <bool INNER, bool BATCH>
 __global__ void __launch_bounds__(GCS_PERF_THREADS, 4)
-vertex_perf_kernel(GcsGraphView G, GcsStateView St, GcsPerfTables T, Ctrl *ctrl_all, const int *__restrict__ vprob, GcsPerfLayout L, PeerPush P) {
+vertex_perf_kernel(GcsGraphView G, GcsStateView St, GcsPerfTables T, Ctrl *ctrl_all, GcsPerfLayout L, PeerPush P) {
     extern __shared__ __align__(16) double smem[];
     __shared__ __align__(8) unsigned long long bar[2];
-    if (!vprob && ctrl_all->stop && !ctrl_all->ignore_stop) return;
+    if (!BATCH) {
+        if (ctrl_all->stop && !ctrl_all->ignore_stop) return;
+        if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&ctrl_all->inner_iters, (unsigned long long)T.inner_iters * (unsigned long long)G.nV);   // K passes over every vertex
+    }
     int tile = blockIdx.x;
     if (tile >= T.ntiles) return;
     double *const stage0 = smem + L.work;
@@ -191,19 +195,14 @@ vertex_perf_kernel(GcsGraphView G, GcsStateView St, GcsPerfTables T, Ctrl *ctrl_
         gcs_perf_stage(T, L, STAGE(0), tile, &bar[0]);
     }
     __syncthreads();                   // the barrier objects are initialised before anybody polls them
-    unsigned phase = 0;                // bit b: parity of the next completion of bar[b]
     double rin = 0.0;                  // INNER: this thread's share of the block's squared inner residual
-    for (int buf = 0; tile < T.ntiles; tile += gridDim.x, buf ^= 1) {
-        const int next = tile + gridDim.x;
-        if (threadIdx.x == 0 && next < T.ntiles) {
-            gcs_bulk_wait_read();      // the stores of the tile that used the other buffer have finished reading it
-            gcs_perf_stage(T, L, STAGE(buf ^ 1), next, &bar[buf ^ 1]);
-        }
-        gcs_mbar_wait(&bar[buf], (phase >> buf) & 1u);
-        phase ^= 1u << buf;
-        gcs_perf_tile<INNER>(G, St, T, L, smem, STAGE(buf), tile, ctrl_all, vprob, rin);
+    for (unsigned n = 0; tile < T.ntiles; tile += gridDim.x, ++n) {
+        const int buf = n & 1;         // the n-th tile of the block is the (n / 2)-th completion of bar[buf]: its parity is (n / 2) & 1
+        gcs_mbar_wait(&bar[buf], (n >> 1) & 1u);
+        // stages tile + gridDim.x into the other buffer once the tile's first barrier is passed
+        gcs_perf_tile<INNER, BATCH>(G, St, T, L, smem, STAGE(buf), tile, ctrl_all, rin, STAGE(buf ^ 1), tile + gridDim.x, &bar[buf ^ 1]);
     }
-    if (threadIdx.x == 0) gcs_bulk_wait_read();   // shared memory stays valid until the last stores have read it
+    if (threadIdx.x == GCS_COPY_THREAD) gcs_bulk_wait_read();   // shared memory stays valid until the last stores have read it
 #undef STAGE
     if (INNER) {     // one partial per thread block, summed in a fixed order (static tile assignment: reproducible run to run)
 #pragma unroll
@@ -928,8 +927,9 @@ static GcsStateView state_view(const GcsHandle *h) {
 static int launch_k1(GcsHandle *h) {
     if (h->perf_on) {
         PeerPush P = {h->send_he, h->send_rank, h->send_slot, h->nsend, h->peer_on ? h->PV_dev : nullptr, h->push_ticket};
-        if (h->inner_on) vertex_perf_kernel<true><<<h->perf_grid, h->perf_threads, h->perf_smem, h->stream>>>(graph_view(h), state_view(h), h->PT, h->ctrl, h->vprob, h->PL, P);
-        else vertex_perf_kernel<false><<<h->perf_grid, h->perf_threads, h->perf_smem, h->stream>>>(graph_view(h), state_view(h), h->PT, h->ctrl, h->vprob, h->PL, P);
+        auto *k = h->vprob ? (h->inner_on ? vertex_perf_kernel<true, true> : vertex_perf_kernel<false, true>)
+                           : (h->inner_on ? vertex_perf_kernel<true, false> : vertex_perf_kernel<false, false>);
+        k<<<h->perf_grid, h->perf_threads, h->perf_smem, h->stream>>>(graph_view(h), state_view(h), h->PT, h->ctrl, h->PL, P);
         return 0;
     }
     vertex_kernel<<<h->k1_blocks, h->k1_warps * 32, h->k1_smem, h->stream>>>(graph_view(h), state_view(h), h->ctrl, h->vprob, h->L, h->p.inner_tol, h->p.inner_max_iter);
@@ -1388,7 +1388,7 @@ extern "C" int gcsadmm_enable_perf(GcsHandle *h, const GcsPerfConfig *c) {
             for (size_t b = 0; b < nB; ++b) {
                 brec[4 * b] = c->blk_he[b]; brec[4 * b + 1] = c->blk_info[b]; brec[4 * b + 2] = c->blk_he[b] >= 0 ? he_edge[c->blk_he[b]] : -1;
             }
-            for (int t = 0; t < c->n_tiles; ++t) {
+            for (int t = 0; t < c->n_tiles && !rc; ++t) {
                 const int a = c->tile_voff[t], b = c->tile_voff[t + 1];
                 int *r = trec + 8 * (size_t)t;
                 r[0] = a; r[1] = b - a; r[2] = c->blk_off[a]; r[3] = c->blk_off[b] - c->blk_off[a];
@@ -1396,15 +1396,22 @@ extern "C" int gcsadmm_enable_perf(GcsHandle *h, const GcsPerfConfig *c) {
                 bool zero = false;
                 for (int hh = he_off[a]; hh < he_off[b]; ++hh) zero = zero || (he_flags[hh] & GCS_HE_FLAG_ZERO);
                 if (zero) r[7] |= 1 << 30;
-                for (int v = a; v < b; ++v) {
+                for (int v = a; v < b && !rc; ++v) {
+                    // the kernel sums the in- and the out-blocks of a vertex as two ranges: in-blocks first, then out-blocks, then its z-block
+                    int nin = 0, g = 0;
+                    for (int bb = c->blk_off[v]; bb < c->blk_off[v + 1]; ++bb) {
+                        const int gb = (c->blk_info[bb] >> 8) & 3;
+                        if (gb < g || (gb == 2) != (bb == c->blk_off[v + 1] - 1)) rc = set_err(GCS_E_INVALID, "perf-mode blocks of a vertex are not in-, out-, z-block order%s", "");
+                        g = gb; nin += gb == 0;
+                    }
                     int *w = vrec + GCS_VI_N * (size_t)v;
                     w[GCS_VI_CONE] = c->cone_off[v] - c->cone_off[a]; w[GCS_VI_NV] = c->cone_off[v + 1] - c->cone_off[v];
-                    w[GCS_VI_CLS] = c->vclass[v]; w[GCS_VI_TERM] = vtype[v] != GCS_VT_GENERIC;
+                    w[GCS_VI_CLS] = c->vclass[v]; w[GCS_VI_TERM] = (vtype[v] != GCS_VT_GENERIC) | (nin << 1);
                     w[GCS_VI_BLK] = c->blk_off[v] - c->blk_off[a]; w[GCS_VI_NB] = c->blk_off[v + 1] - c->blk_off[v];
                     w[GCS_VI_ACTIVE] = vprob[v]; w[GCS_VI_HE] = he_off[v] - he_off[a];
                 }
             }
-            rc = upload(&h->p_blk_rec, brec, 4 * nB);
+            if (!rc) rc = upload(&h->p_blk_rec, brec, 4 * nB);
             if (!rc) rc = upload(&h->p_vrec, vrec, GCS_VI_N * nVt);
             if (!rc) rc = upload(&h->p_tile_rec, trec, 8 * nT);
         }
@@ -1436,10 +1443,10 @@ extern "C" int gcsadmm_enable_perf(GcsHandle *h, const GcsPerfConfig *c) {
         const long long cap = (long long)prop.multiProcessorCount * per_sm;
         h->perf_grid = (int)(c->n_tiles < cap ? c->n_tiles : cap);
     }
-    CK(cudaFuncSetAttribute(vertex_perf_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->perf_smem));
-    CK(cudaFuncSetAttribute(vertex_perf_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    CK(cudaFuncSetAttribute(vertex_perf_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->perf_smem));
-    CK(cudaFuncSetAttribute(vertex_perf_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+    for (auto *k : {vertex_perf_kernel<false, false>, vertex_perf_kernel<true, false>, vertex_perf_kernel<false, true>, vertex_perf_kernel<true, true>}) {
+        CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, h->perf_smem));
+        CK(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+    }
     perf_init_dead_kernel<<<(h->nV + 255) / 256, 256, 0, h->stream>>>(graph_view(h), state_view(h));
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(h->stream));

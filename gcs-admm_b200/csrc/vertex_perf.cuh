@@ -55,7 +55,7 @@ struct GcsPerfTables {
     const double *cls_tab;     // [ncls][GCS_CLS_STRIDE]
     const int *cone_off;       // [nV+1] polygon vertices of vertex v: cone_off[v]..cone_off[v+1]
     const double *cone;        // GCS_CONE_REC doubles per polygon vertex (see gcs_cone_project)
-    const int *blk_off;        // [nV+1] blocks of vertex v: its live half-edges in half-edge order, then (z_v, y_v)
+    const int *blk_off;        // [nV+1] blocks of vertex v: its live half-edges in half-edge order (in-half-edges first), then (z_v, y_v)
     const int *blk_rec;        // [B][4]: half-edge of the block (-1 for the (z_v, y_v) block) | descriptor: bits 0-7 vertex index inside its
                                //         tile, bits 8-9 group (0 in, 1 out, 2 z-block), bit 10 's' / 't' | edge of the half-edge | 0
     const int *vrec;           // [nV][GCS_VI_N]: the per-vertex descriptor the kernel keeps in shared memory (offsets relative to the tile)
@@ -81,7 +81,7 @@ struct GcsPerfLayout { int nb_cap, nvt_cap, cone_cap, tS, cone, tnS, vi, bi, tr,
 #define GCS_VI_CONE 0     // first cone record, relative to the tile's
 #define GCS_VI_NV 1       // polygon vertices
 #define GCS_VI_CLS 2
-#define GCS_VI_TERM 3
+#define GCS_VI_TERM 3     // bit 0: 's' / 't' vertex | bits 1-: live in-half-edges (its blocks hold all of them before any out-half-edge)
 #define GCS_VI_BLK 4      // first block, relative to the tile's
 #define GCS_VI_NB 5       // blocks (0: dead vertex)
 #define GCS_VI_ACTIVE 6   // its problem is still iterating (the table holds the vertex's problem index here)
@@ -123,30 +123,39 @@ static inline GcsPerfLayout gcs_perf_layout(int nb_cap, int nvt_cap, int cone_ca
 // face's sector: unique, and no other candidate can be nearer), on a ray (the one with the largest reduction
 // tau^2 / |r|^2 of the squared distance), or is the apex.  ma, mb are orthogonal to n_k, so the sector test of the foot
 // point  c - dist n_k  is a test on c itself.
-GCS_DEV void gcs_cone_project(const double *cone, int nv, double c0, double c1, double c2, double &q0, double &q1, double &q2) {
-    double best = 0.0;
-    int code = -1;          // -1 apex | 2k ray k | 2k+1 face k
-    bool inside = true;
-    for (int k = 0; k < nv; ++k) {
+// record k: ray and face (read for every record); the sector normals are read only when a point is outside face k
+struct GcsConeRay { double vx, vy, nx, ny, nh, inv; };
 #if defined(GCS_EMULATE)
-        const double *r = cone + GCS_CONE_REC * k;
-        const double vx = r[0], vy = r[1], nx = r[2], ny = r[3], nh = r[4], inv = r[5], a0 = r[6], a1 = r[7], a2 = r[8], b0 = r[9], b1 = r[10], b2 = r[11];
+GCS_DEV GcsConeRay gcs_cone_ray(const double *cone, int k) { const double *r = cone + GCS_CONE_REC * k; return GcsConeRay{r[0], r[1], r[2], r[3], r[4], r[5]}; }
 #else
-        const double2 *r = reinterpret_cast<const double2 *>(cone + GCS_CONE_REC * k);     // records are 96 bytes, 16-byte aligned: 6 LDS.128
-        const double2 r0 = r[0], r1 = r[1], r2 = r[2], r3 = r[3], r4 = r[4], r5 = r[5];
-        const double vx = r0.x, vy = r0.y, nx = r1.x, ny = r1.y, nh = r2.x, inv = r2.y, a0 = r3.x, a1 = r3.y, a2 = r4.x, b0 = r4.y, b1 = r5.x, b2 = r5.y;
+// records are 96 bytes, 16-byte aligned: 3 LDS.128 for the ray and the face, 2 + 2 for the sector normals
+GCS_DEV GcsConeRay gcs_cone_ray(const double *cone, int k) {
+    const double2 *r = reinterpret_cast<const double2 *>(cone + GCS_CONE_REC * k);
+    const double2 r0 = r[0], r1 = r[1], r2 = r[2];
+    return GcsConeRay{r0.x, r0.y, r1.x, r1.y, r2.x, r2.y};
+}
 #endif
-        const double tau = c0 * vx + c1 * vy + c2;
-        const double dist = nx * c0 + ny * c1 + nh * c2;
-        if (tau > 0.0) {
-            const double red = tau * tau * inv;
-            if (red > best) { best = red; code = 2 * k; }
-        }
-        if (dist > 0.0) {
-            inside = false;
-            if (c0 * a0 + c1 * a1 + c2 * a2 >= 0.0 && c0 * b0 + c1 * b1 + c2 * b2 >= 0.0) { best = 1e300; code = 2 * k + 1; }
-        }
+// sector normal ma (s = 0) or mb (s = 1) of record k dotted with the point c
+GCS_DEV double gcs_cone_sector_dot(const double *cone, int k, int s, double c0, double c1, double c2) {
+    const double *m = cone + GCS_CONE_REC * k + 6 + 3 * s;
+    return c0 * m[0] + c1 * m[1] + c2 * m[2];
+}
+// candidate ray k for the point c (code: -1 apex | 2k ray k | 2k+1 face k); returns the signed distance of c from face k
+GCS_DEV double gcs_cone_test_ray(const GcsConeRay &R, int k, double c0, double c1, double c2, double &best, int &code) {
+    const double tau = c0 * R.vx + c1 * R.vy + c2;
+    const double dist = R.nx * c0 + R.ny * c1 + R.nh * c2;
+    if (tau > 0.0) {
+        const double red = tau * tau * R.inv;
+        if (red > best) { best = red; code = 2 * k; }
     }
+    return dist;
+}
+// face k is the candidate for a point c outside it (dist > 0) whose dot products with both sector normals are >= 0
+GCS_DEV void gcs_cone_take_face(bool sector, int k, double &best, int &code, bool &inside) {
+    inside = false;
+    if (sector) { best = 1e300; code = 2 * k + 1; }
+}
+GCS_DEV void gcs_cone_pick(const double *cone, int code, bool inside, double c0, double c1, double c2, double &q0, double &q1, double &q2) {
     if (inside) { q0 = c0; q1 = c1; q2 = c2; return; }
     q0 = 0.0; q1 = 0.0; q2 = 0.0;
     if (code < 0) return;
@@ -158,6 +167,40 @@ GCS_DEV void gcs_cone_project(const double *cone, int nv, double c0, double c1, 
         const double tau = (c0 * ck[0] + c1 * ck[1] + c2) * ck[5];
         q0 = tau * ck[0]; q1 = tau * ck[1]; q2 = tau;
     }
+}
+GCS_DEV void gcs_cone_project(const double *cone, int nv, double c0, double c1, double c2, double &q0, double &q1, double &q2) {
+    double best = 0.0;
+    int code = -1;
+    bool inside = true;
+#pragma unroll 1
+    for (int k = 0; k < nv; ++k) {
+        const double dist = gcs_cone_test_ray(gcs_cone_ray(cone, k), k, c0, c1, c2, best, code);
+        if (dist > 0.0) gcs_cone_take_face(gcs_cone_sector_dot(cone, k, 0, c0, c1, c2) >= 0.0 && gcs_cone_sector_dot(cone, k, 1, c0, c1, c2) >= 0.0, k, best, code, inside);
+    }
+    gcs_cone_pick(cone, code, inside, c0, c1, c2, q0, q1, q2);
+}
+// the same projection of two points onto one cone: each record is loaded once for both points (two independent dependency
+// chains); every point sees exactly the expressions of gcs_cone_project in the same order, so the results are bit-identical to
+// two calls
+GCS_DEV void gcs_cone_project2(const double *cone, int nv, double c0, double c1, double c2, double d0, double d1, double d2,
+                               double &q0, double &q1, double &q2, double &s0, double &s1, double &s2) {
+    double best_c = 0.0, best_d = 0.0;
+    int code_c = -1, code_d = -1;
+    bool inside_c = true, inside_d = true;
+#pragma unroll 1
+    for (int k = 0; k < nv; ++k) {
+        const GcsConeRay R = gcs_cone_ray(cone, k);
+        const double dist_c = gcs_cone_test_ray(R, k, c0, c1, c2, best_c, code_c);
+        const double dist_d = gcs_cone_test_ray(R, k, d0, d1, d2, best_d, code_d);
+        if (dist_c > 0.0 || dist_d > 0.0) {      // the sector normals one at a time: fewer registers live
+            const bool ma_c = gcs_cone_sector_dot(cone, k, 0, c0, c1, c2) >= 0.0, ma_d = gcs_cone_sector_dot(cone, k, 0, d0, d1, d2) >= 0.0;
+            const bool mb_c = gcs_cone_sector_dot(cone, k, 1, c0, c1, c2) >= 0.0, mb_d = gcs_cone_sector_dot(cone, k, 1, d0, d1, d2) >= 0.0;
+            if (dist_c > 0.0) gcs_cone_take_face(ma_c && mb_c, k, best_c, code_c, inside_c);
+            if (dist_d > 0.0) gcs_cone_take_face(ma_d && mb_d, k, best_d, code_d, inside_d);
+        }
+    }
+    gcs_cone_pick(cone, code_c, inside_c, c0, c1, c2, q0, q1, q2);
+    gcs_cone_pick(cone, code_d, inside_d, d0, d1, d2, s0, s1, s2);
 }
 
 #if !defined(GCS_EMULATE) && defined(__CUDACC__)
@@ -192,15 +235,15 @@ __device__ __forceinline__ void gcs_fence_async_smem() { asm volatile("fence.pro
 #define GCS_PF 3   // consensus targets a thread keeps in registers between issuing their loads and using them (device build)
 
 // input k of the extended core of vertex vl:  r_x (4) | r_z, r_yv (5) | sum of r over the in-blocks (5) | over the out-blocks (5)
-GCS_DEV double gcs_core_input(const double *tS, const double *rS, const int *brec, const int *w, int k, double kappa) {
+GCS_DEV double gcs_core_input(const double *tS, const double *rS, const int *w, int k, double kappa) {
     const int bl = w[GCS_VI_BLK], zb = bl + w[GCS_VI_NB] - 1;
     double s = 0.0;
     if (k < 4) {
-        if (!w[GCS_VI_TERM]) { for (int b = bl; b <= zb; ++b) s += tS[12 * b + 6 * (k >> 1) + 3 + (k & 1)]; s *= kappa; }
+        if (!(w[GCS_VI_TERM] & 1)) { for (int b = bl; b <= zb; ++b) s += tS[12 * b + 6 * (k >> 1) + 3 + (k & 1)]; s *= kappa; }
     } else if (k < 9) s = rS[5 * zb + k - 4];
-    else {
-        const int g = k >= 14, tau = k - 9 - 5 * g;
-        for (int b = bl; b < zb; ++b) if (((brec[4 * b + 1] >> 8) & 3) == g) s += rS[5 * b + tau];
+    else {      // the in-blocks are bl .. bl + nin - 1, the out-blocks follow up to the z-block
+        const int g = k >= 14, tau = k - 9 - 5 * g, bin = bl + (w[GCS_VI_TERM] >> 1);
+        for (int b = g ? bin : bl; b < (g ? zb : bin); ++b) s += rS[5 * b + tau];
     }
     return s;
 }
@@ -251,7 +294,11 @@ GCS_DEV double gcs_target_z(const GcsStateView &St, const GcsPerfTables &T, int 
     return zc;
 }
 
+
 #if !defined(GCS_EMULATE) && defined(__CUDACC__)
+// the thread that issues and waits for the bulk copies of the tiles after the first (bulk groups belong to the thread that
+// commits them): lane 0 of the last warp, which has no vertex in P3 - P5 when a tile has fewer vertices than the block has warps
+#define GCS_COPY_THREAD (blockDim.x - 32)
 // P0 (one thread): the bulk copies that stage tile `tile` into the stage buffer B; completion is signalled on `bar`
 __device__ __forceinline__ void gcs_perf_stage(const GcsPerfTables &T, const GcsPerfLayout &L, double *B, int tile, unsigned long long *bar) {
     const int *tr = T.tile_rec + 8 * (size_t)tile;
@@ -266,21 +313,33 @@ __device__ __forceinline__ void gcs_perf_stage(const GcsPerfTables &T, const Gcs
 }
 #endif
 
+// c-step of one pair from its projection q:  d = c - lam replaces t in place, e = (1 - alpha) c + lam waits for the t-step
+GCS_DEV void gcs_cstep_store(double *t, double *e, double t0, double t1, double t2, double q0, double q1, double q2, double ms, double alpha) {
+    const double l0 = ms * (t0 - q0), l1 = ms * (t1 - q1), l2 = ms * (t2 - q2);
+    t[0] = q0 - l0; t[1] = q1 - l1; t[2] = q2 - l2;
+    e[0] = (1.0 - alpha) * q0 + l0; e[1] = (1.0 - alpha) * q1 + l1; e[2] = (1.0 - alpha) * q2 + l2;
+}
+
 // x-update of one tile of vertices in perf mode.  S: work arrays, B: the tile's staged arrays (device build: already filled by
-// gcs_perf_stage and waited for; the new state leaves B by bulk stores that the CALLER waits for before B is refilled).
+// gcs_perf_stage and waited for; the new state leaves B by bulk stores of GCS_COPY_THREAD).  Device build: after the tile's first
+// barrier GCS_COPY_THREAD waits until the stores of the previous tile have read Bn and stages tile `next` into it (signalled on
+// bar_next): the stores drain during P1 - P2 and the loads land during P3 - P8, without holding the block at a barrier.
 // INNER: also accumulate (into `rin`, per thread) the squared inner residual  |(M u + m0) - c|^2  of the tile's pairs after the
 // last pass — compiled in only for the kernel variant the host switches to near convergence (gcsadmm_run), so the throughput
 // path carries none of it.
-template <bool INNER>
+// BATCH: the tile's vertices belong to several problems, each with its own control block ctrl_all[GCS_VI_ACTIVE of the vertex]
+// (rho, mu_scale, stop flag per vertex); otherwise one problem, ctrl_all.
+template <bool INNER, bool BATCH>
 GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const GcsPerfTables &T, const GcsPerfLayout &L,
-                           double *S, double *B, int tile, Ctrl *ctrl_all, const int *vprob, double &rin) {
+                           double *S, double *B, int tile, Ctrl *ctrl_all, double &rin,
+                           double *Bn, int next, unsigned long long *bar_next) {
     // single problem: rho / mu_scale are uniform — loaded once into registers here
     // (batched problems: per vertex, from its problem's control block)
     const double rho_u = ctrl_all->rho, ms_u = ctrl_all->mu_scale;
-#define RHO(vl) (vprob ? vd[2 * (vl)] : rho_u)
-#define MSC(vl) (vprob ? vd[2 * (vl) + 1] : ms_u)
-#define ACT(vl) (!vprob || vi[GCS_VI_N * (vl) + GCS_VI_ACTIVE])
-#define ACT_W (!vprob || w[GCS_VI_ACTIVE])
+#define RHO(vl) (BATCH ? vd[2 * (vl)] : rho_u)
+#define MSC(vl) (BATCH ? vd[2 * (vl) + 1] : ms_u)
+#define ACT(vl) (!BATCH || vi[GCS_VI_N * (vl) + GCS_VI_ACTIVE])
+#define ACT_W (!BATCH || w[GCS_VI_ACTIVE])
 #if defined(GCS_EMULATE)
     const int *tr = T.tile_rec + 8 * (size_t)tile;
 #else
@@ -304,7 +363,18 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
         memcpy(brec, T.blk_rec + 4 * (size_t)b0, sizeof(int) * 4 * nb);
     }
 #endif
-    if (vprob) {
+    // Until the first barrier of a pass the block works as two groups: the first half of the warps does the c-step, two pairs per
+    // thread; the others issue the gathers of the consensus targets, answer the forced-zero half-edges and do the path-length item
+    // meanwhile.  A one-warp block does both, one after the other.
+#if defined(GCS_EMULATE)
+    const bool cgrp = true, ggrp = true;
+    const int cid = 0, cn = 1, gid0 = 0, gn = 1;
+#else
+    const int nw = blockDim.x >> 5, cn = 32 * ((nw + 1) >> 1);
+    const bool cgrp = (int)threadIdx.x < cn, ggrp = !cgrp || nw == 1;
+    const int cid = threadIdx.x, gid0 = nw == 1 ? (int)threadIdx.x : (int)threadIdx.x - cn, gn = nw == 1 ? cn : (int)blockDim.x - cn;
+#endif
+    if (BATCH) {
         GCS_CTA_LOOP(i, nvt) {     // rho, mu_scale and the stop flag of the vertex's problem
             int *w = vi + GCS_VI_N * i;
             Ctrl *c = ctrl_all + w[GCS_VI_ACTIVE];
@@ -318,79 +388,102 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
 #endif
             }
         }
-    }
-    // ---- P1: consensus targets  T = z_e + mu_h  of the live half-edges.  Device build: the gathers are only ISSUED here — the
-    // values stay in registers while the thread does its cone projections and are combined after them, so the DRAM / L2
-    // latency of the gather hides behind the c-step instead of stalling the block; forced-zero half-edges are answered directly
-#if !defined(GCS_EMULATE)
-    double pz[GCS_PF], pm[GCS_PF];
-#pragma unroll
-    for (int j = 0; j < GCS_PF; ++j) {
-        const int q = threadIdx.x + j * blockDim.x;
-        pz[j] = 0.0; pm[j] = 0.0;
-        if (q < 5 * nb) {
-            const int b = q / 5, c = q - 5 * b, h = bhe(b);
-            if (h >= 0) { pz[j] = gcs_target_z(St, T, bedge(b), c, binfo(b)); pm[j] = St.mu[5 * (size_t)h + c]; }
-        }
-    }
-#endif
-    if (vprob) GCS_CTA_SYNC();     // vd / ACTIVE of every vertex of the tile are in shared memory
-    if (has_zero) GCS_CTA_LOOP(q, 5 * nhe) {
-        const int hl = q / 5, c = q - 5 * hl, h = h0 + hl, f = G.he_flags[h];
-        if (!(f & GCS_HE_ZERO)) continue;
-        int vl = 0;
-        while (vl + 1 < nvt && vi[GCS_VI_N * (vl + 1) + GCS_VI_HE] <= hl) ++vl;
-        if (!ACT(vl)) continue;
-        // own copy and flow are 0; an incoming edge's "other copy" first point is unconstrained and sits on its target
-        double x = 0.0;
-        if (c < 2 && !(f & GCS_HE_OUT)) x = St.z[5 * (size_t)G.he_edge[h] + c] + MSC(vl) * St.mu[5 * (size_t)h + c];
-        St.xc[5 * (size_t)h + c] = x;
+        GCS_CTA_SYNC();     // vd / ACTIVE of every vertex of the tile are in shared memory
     }
     const double alpha = T.alpha, kappa = T.kappa;
     for (int it = 0; it < T.inner_iters; ++it) {
         const bool last = it + 1 == T.inner_iters;
-        // ---- P2: c-step.  d = c - lam (what the v-step sees) replaces t in place; e = (1 - alpha) c + lam waits for the t-step
-        GCS_CTA_LOOP(p, 4 * nb) {
-            const int b = p >> 2, info = binfo(b), vl = info & 255;
-            const int *w = vi + GCS_VI_N * vl;
-            if (!ACT_W || ((info >> 10) & (p & 1))) continue;       // 's' / 't' have no C2 / C4 pairs
-            const double ms = it ? 1.0 : MSC(vl);                      // sigma = kappa rho: lam rescales with mu (:705 / :708)
-            double *t = tS + 3 * p, *e = eS + 3 * p;
-            const double t0 = t[0], t1 = t[1], t2 = t[2];
-            double q0, q1, q2;
-            gcs_cone_project(coneS + GCS_CONE_REC * w[GCS_VI_CONE], w[GCS_VI_NV], t0, t1, t2, q0, q1, q2);
-            const double l0 = ms * (t0 - q0), l1 = ms * (t1 - q1), l2 = ms * (t2 - q2);
-            t[0] = q0 - l0; t[1] = q1 - l1; t[2] = q2 - l2;
-            e[0] = (1.0 - alpha) * q0 + l0; e[1] = (1.0 - alpha) * q1 + l1; e[2] = (1.0 - alpha) * q2 + l2;
-        }
-        GCS_CTA_LOOP(i, nvt) {                                                // path-length item: block soft-threshold, threshold 1 / sigma
-            const int *w = vi + GCS_VI_N * i;
-            if (!ACT_W || !w[GCS_VI_NB]) continue;
-            const double ms = it ? 1.0 : MSC(i);
-            const double sigma = kappa * RHO(i) * ms;                      // the threshold of the pass that produced t (rho before its rescale)
-            const double a0 = tnS[2 * i], a1 = tnS[2 * i + 1], nrm = hypot(a0, a1);
-            const double sc = nrm > 0.0 ? fmax(0.0, 1.0 - 1.0 / (sigma * nrm)) : 0.0;
-            const double q0 = sc * a0, q1 = sc * a1, l0 = ms * (a0 - q0), l1 = ms * (a1 - q1);
-            tnS[2 * i] = q0 - l0; tnS[2 * i + 1] = q1 - l1;
-            enS[2 * i] = (1.0 - alpha) * q0 + l0; enS[2 * i + 1] = (1.0 - alpha) * q1 + l1;
-        }
-        if (it == 0) {        // the targets whose loads were issued in P1
+        if (ggrp) {
+#if defined(GCS_EMULATE)
+            const int gid = gid0;
+#else
+            // opaque inside the pass: otherwise the gather slots' block / scalar indices are hoisted out of the tile and pass
+            // loops and held in registers through every phase (spills at 64 registers)
+            int gid = gid0;
+            asm volatile("" : "+r"(gid));
+#endif
+            if (it == 0 && has_zero) for (int q = gid; q < 5 * nhe; q += gn) {
+                const int hl = q / 5, c = q - 5 * hl, h = h0 + hl, f = G.he_flags[h];
+                if (!(f & GCS_HE_ZERO)) continue;
+                int vl = 0;
+                while (vl + 1 < nvt && vi[GCS_VI_N * (vl + 1) + GCS_VI_HE] <= hl) ++vl;
+                if (!ACT(vl)) continue;
+                // own copy and flow are 0; an incoming edge's "other copy" first point is unconstrained and sits on its target
+                double x = 0.0;
+                if (c < 2 && !(f & GCS_HE_OUT)) x = St.z[5 * (size_t)G.he_edge[h] + c] + MSC(vl) * St.mu[5 * (size_t)h + c];
+                St.xc[5 * (size_t)h + c] = x;
+            }
+            for (int i = gid; i < nvt; i += gn) {                           // path-length item: block soft-threshold, threshold 1 / sigma
+                const int *w = vi + GCS_VI_N * i;
+                if (!ACT_W || !w[GCS_VI_NB]) continue;
+                const double ms = it ? 1.0 : MSC(i);
+                const double sigma = kappa * RHO(i) * ms;                      // the threshold of the pass that produced t (rho before its rescale)
+                const double a0 = tnS[2 * i], a1 = tnS[2 * i + 1], nrm = hypot(a0, a1);
+                const double sc = nrm > 0.0 ? fmax(0.0, 1.0 - 1.0 / (sigma * nrm)) : 0.0;
+                const double q0 = sc * a0, q1 = sc * a1, l0 = ms * (a0 - q0), l1 = ms * (a1 - q1);
+                tnS[2 * i] = q0 - l0; tnS[2 * i + 1] = q1 - l1;
+                enS[2 * i] = (1.0 - alpha) * q0 + l0; enS[2 * i + 1] = (1.0 - alpha) * q1 + l1;
+            }
+            // ---- P1 (first pass): consensus targets  T = z_e + mu_h  of the live half-edges.  Device build: the GCS_PF gathers of a
+            // thread are all issued before the first is used (their DRAM / L2 latency overlaps), while the other warps project
+#if !defined(GCS_EMULATE)
+            double pz[GCS_PF], pm[GCS_PF];
+            if (it == 0) {
+#pragma unroll
+                for (int j = 0; j < GCS_PF; ++j) {
+                    const int q = gid + j * gn;
+                    pz[j] = 0.0; pm[j] = 0.0;
+                    if (q < 5 * nb) {
+                        const int b = q / 5, c = q - 5 * b, h = bhe(b);
+                        if (h >= 0) { pz[j] = gcs_target_z(St, T, bedge(b), c, binfo(b)); pm[j] = St.mu[5 * (size_t)h + c]; }
+                    }
+                }
+            }
+#endif
+            if (it == 0) {
 #if !defined(GCS_EMULATE)
 #pragma unroll
-            for (int j = 0; j < GCS_PF; ++j) {
-                const int q = threadIdx.x + j * blockDim.x;
-                if (q < 5 * nb) TS[q] = pz[j] + MSC(binfo(q / 5) & 255) * pm[j];
-            }
-            for (int q = threadIdx.x + GCS_PF * blockDim.x; q < 5 * nb; q += blockDim.x) {
+                for (int j = 0; j < GCS_PF; ++j) {
+                    const int q = gid + j * gn;
+                    if (q < 5 * nb) TS[q] = pz[j] + MSC(binfo(q / 5) & 255) * pm[j];
+                }
+                for (int q = gid + GCS_PF * gn; q < 5 * nb; q += gn) {     // small blocks: the targets beyond the prefetched ones
 #else
-            for (int q = 0; q < 5 * nb; ++q) {
+                for (int q = 0; q < 5 * nb; ++q) {
 #endif
-                const int b = q / 5, c = q - 5 * b, h = bhe(b), vl = binfo(b) & 255;
-                if (h < 0 || !ACT(vl)) continue;
-                TS[q] = gcs_target_z(St, T, bedge(b), c, binfo(b)) + MSC(vl) * St.mu[5 * (size_t)h + c];
+                    const int b = q / 5, c = q - 5 * b, h = bhe(b), vl = binfo(b) & 255;
+                    if (h < 0 || !ACT(vl)) continue;
+                    TS[q] = gcs_target_z(St, T, bedge(b), c, binfo(b)) + MSC(vl) * St.mu[5 * (size_t)h + c];
+                }
             }
         }
+        // ---- P2: c-step.  Item j = point i of block b (j = 2 b + i): its fam-0 and fam-1 pairs p = 2 j, 2 j + 1 belong to one vertex
+        // and are projected onto its cone in one pass over the records ('s' / 't' blocks have no fam-1 pair: no C2 / C4)
+        if (cgrp) for (int j = cid; j < 2 * nb; j += cn) {
+            const int b = j >> 1, info = binfo(b), vl = info & 255;
+            const int *w = vi + GCS_VI_N * vl;
+            if (!ACT_W) continue;
+            const double ms = it ? 1.0 : MSC(vl);                      // sigma = kappa rho: lam rescales with mu (:705 / :708)
+            const double *cone = coneS + GCS_CONE_REC * w[GCS_VI_CONE];
+            double *t = tS + 6 * j, *e = eS + 6 * j;
+            const double t0 = t[0], t1 = t[1], t2 = t[2];
+            double q0, q1, q2;
+            if ((info >> 10) & 1) gcs_cone_project(cone, w[GCS_VI_NV], t0, t1, t2, q0, q1, q2);
+            else {
+                const double t3 = t[3], t4 = t[4], t5 = t[5];
+                double q3, q4, q5;
+                gcs_cone_project2(cone, w[GCS_VI_NV], t0, t1, t2, t3, t4, t5, q0, q1, q2, q3, q4, q5);
+                gcs_cstep_store(t + 3, e + 3, t3, t4, t5, q3, q4, q5, ms, alpha);
+            }
+            gcs_cstep_store(t, e, t0, t1, t2, q0, q1, q2, ms, alpha);
+        }
         GCS_CTA_SYNC();
+#if !defined(GCS_EMULATE)
+        if (it == 0 && threadIdx.x == GCS_COPY_THREAD && next < T.ntiles) {
+            gcs_bulk_wait_read();      // the stores of the previous tile have finished reading Bn
+            gcs_perf_stage(T, L, Bn, next, bar_next);
+        }
+#endif
         // ---- P3 + P4 + P5, one warp per vertex (device build), so that only warp barriers separate them:
         //   P3  right-hand side of the v-step in units of rho,  r = S'T - (eps / rho) e_y + kappa M'(d - m0),  for the vertex's blocks
         //   P4  the 19 inputs of its extended core (r_x, r_z, r_yv, sums of r over the in- and the out-blocks)
@@ -400,7 +493,7 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
             const int *w = vi + GCS_VI_N * vl;
             if (!ACT_W || !w[GCS_VI_NB]) continue;
             for (int q = 5 * w[GCS_VI_BLK]; q < 5 * (w[GCS_VI_BLK] + w[GCS_VI_NB]); ++q) rS[q] = gcs_rhs(T, tS, TS, tnS, brec, q, vl, RHO(vl), kappa);
-            for (int k = 0; k < GCS_NCX; ++k) cin[GCS_NCX * vl + k] = gcs_core_input(tS, rS, brec, w, k, kappa);
+            for (int k = 0; k < GCS_NCX; ++k) cin[GCS_NCX * vl + k] = gcs_core_input(tS, rS, w, k, kappa);
             for (int k = 0; k < GCS_NCX; ++k) cout[GCS_NCX * vl + k] = gcs_core_output(T.cls_tab + (size_t)GCS_CLS_STRIDE * w[GCS_VI_CLS], cin + GCS_NCX * vl, k);
         }
 #else
@@ -410,7 +503,7 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
             if (!ACT_W || !w[GCS_VI_NB]) continue;                    // warp-uniform
             for (int q = 5 * w[GCS_VI_BLK] + k; q < 5 * (w[GCS_VI_BLK] + w[GCS_VI_NB]); q += 32) rS[q] = gcs_rhs(T, tS, TS, tnS, brec, q, vl, RHO(vl), kappa);
             __syncwarp();
-            if (k < GCS_NCX) cin[GCS_NCX * vl + k] = gcs_core_input(tS, rS, brec, w, k, kappa);
+            if (k < GCS_NCX) cin[GCS_NCX * vl + k] = gcs_core_input(tS, rS, w, k, kappa);
             __syncwarp();
             if (k < GCS_NCX) cout[GCS_NCX * vl + k] = gcs_core_output(T.cls_tab + (size_t)GCS_CLS_STRIDE * w[GCS_VI_CLS], cin + GCS_NCX * vl, k);
         }
@@ -466,19 +559,17 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
         }
         if (!last) GCS_CTA_SYNC();     // (after the last pass P8's barrier follows)
     }
-    // ---- P8: the new state goes back with bulk stores (the caller waits for them before it refills B)
+    // ---- P8: the new state goes back with bulk stores (GCS_COPY_THREAD waits for them before it restages B)
 #if defined(GCS_EMULATE)
     memcpy(T.tstate + 12 * (size_t)b0, tS, sizeof(double) * 12 * nb);
     memcpy(T.tn + 2 * (size_t)v0, tnS, sizeof(double) * 2 * nvt);
-    if (!vprob) ctrl_all->inner_iters += (unsigned long long)T.inner_iters * (unsigned long long)nvt;
 #else
     gcs_fence_async_smem();
     GCS_CTA_SYNC();
-    if (threadIdx.x == 0) {
+    if (threadIdx.x == GCS_COPY_THREAD) {
         if (nb) gcs_bulk_s2g(T.tstate + 12 * (size_t)b0, tS, (unsigned)(sizeof(double) * 12 * nb));
         gcs_bulk_s2g(T.tn + 2 * (size_t)v0, tnS, (unsigned)(sizeof(double) * 2 * nvt));
         gcs_bulk_commit();
-        if (!vprob) atomicAdd(&ctrl_all->inner_iters, (unsigned long long)T.inner_iters * (unsigned long long)nvt);
     }
 #endif
 #undef bhe

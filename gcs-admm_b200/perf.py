@@ -328,6 +328,9 @@ def perf_tables(g, kappa=1.0, cone=None, theta=1.0, frames="global", edge_delta=
     blk_he[blk_off[owner[hl]] + rank_in_v] = hl
     grp = np.full(Btot, 2, dtype=np.int64)
     grp[blk_off[owner[hl]] + rank_in_v] = outm[hl].astype(np.int64)
+    # the kernel sums a vertex's in-blocks and out-blocks as two contiguous ranges: in-blocks first, then out-blocks, then the z-block
+    if Btot and not np.all((np.diff(grp) >= 0) | (np.diff(blk_v) != 0)):
+        raise ValueError("perf tables need every vertex's in-half-edges before its out-half-edges")
     # tiles: greedy over consecutive vertices
     he_cnt = np.diff(np.asarray(g.he_off, dtype=np.int64))
     cone_cnt = np.diff(np.asarray(cone_off, dtype=np.int64))

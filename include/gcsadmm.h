@@ -179,7 +179,8 @@ typedef struct GcsPerfConfig {
     const double *cone;          /* 12 doubles per polygon vertex: Vx, Vy, unit outward normal (3) of the cone face to the
                                     next vertex's ray, 1 / (Vx^2 + Vy^2 + 1), the face's two in-plane sector normals (3 + 3) */
     int32_t n_blocks;            /* blocks = live half-edges + one (z_v, y_v) block per live vertex */
-    const int32_t *blk_off;      /* [nV+1] */
+    const int32_t *blk_off;      /* [nV+1]; a vertex's blocks are its in-blocks, then its out-blocks, then its z-block
+                                    (any other order is refused with GCS_E_INVALID) */
     const int32_t *blk_he;       /* [n_blocks] half-edge of the block, -1 for the (z_v, y_v) block */
     const int32_t *blk_info;     /* [n_blocks] bits 0-7 vertex index inside its tile | 8-9 group (0 in, 1 out, 2 z-block) | 10 terminal */
     int32_t n_tiles;             /* a tile = the consecutive vertices one thread block works on */
