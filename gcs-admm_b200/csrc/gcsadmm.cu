@@ -8,7 +8,8 @@
 //                            atomics on the data), and the LAST block to finish reduces them in a fixed order and applies the
 //                            control step: residuals, rho adaptation, stop rule, history (reference admm_solver_v3.py:697-713)
 //       edge_frames_kernel   the same with one thread per edge: partitions with ghost slots (multi-GPU), the check variant that
-//                            also evaluates the residuals in global coordinates; edge_kernel: one thread per (edge, scalar)
+//                            also evaluates the residuals in global coordinates
+//       batched_edge_kernel  packed independent problems: one block per problem, its own control step
 //   control_kernel           the same control step as a separate launch (NCCL multi-GPU: the sums are all-reduced in between);
 //   peer_control_kernel      peer-memory multi-GPU: waits for every rank's sums, then the control step
 // Every kernel returns immediately once the stop flag is set, so the host can enqueue iterations in
@@ -88,14 +89,14 @@ struct GcsHandle {
     long long n_x, n_mu;
     int dcap, mcap;
     GcsScratchLayout L;
-    int k1_smem, k1_blocks, k1_warps, edge_blocks, edge_per_edge, edge_minb, edge_coop, coop_blocks;
+    int k1_smem, k1_blocks, k1_warps, edge_blocks, edge_coop, coop_blocks;
     // device
     int *poly_off, *he_off, *he_edge, *edge_he_tail, *edge_he_head;
     double *polyA, *polyb, *cent;
     unsigned char *he_flags, *vtype, *edge_counted;
     int *vprob, *prob_eoff; long long *prob_nx, *prob_nmu;   // batched mode (nP > 1)
     int *he_prob_host;  // host: problem of each half-edge (batched mode)
-    unsigned int *ticket;   // edge_kernel: blocks finished in the current launch (the last one reduces + controls)
+    unsigned int *ticket;   // edge kernels: blocks finished in the current launch (the last one reduces + controls)
     unsigned int *push_ticket;   // perf K1 in peer mode: blocks finished (the last one pushes the halo)
     double *xc, *mu, *z, *x_v, *z_v, *y_v;
     double *ws;         // [nV][gcs_ws_stride] interior-point warm-start records (null when warm_theta == 0)
@@ -346,54 +347,61 @@ __device__ __forceinline__ void edge_finish(double r2, double dz2, double x2, do
 // z_e = 1/2 (xc_tail + xc_head)            reference admm_solver_v3.py:543-562 (live scalars only)
 // mu_h <- mu_scale * mu_h + (z_e - xc_h)    :590-594  (mu_scale carries the rho-adaptation rescale :705/:708)
 // partial sums of |z - xc|^2, |dz|^2, |xc|^2, |z|^2, |mu|^2     :597-614
-// One thread per (edge, consensus scalar): z and the tail-side records are walked sequentially (edges are sorted by
-// (tail, head) and a vertex's outgoing half-edges follow that order), the head-side record is a 40-byte gather.
-// oalpha != 1 (perf mode only) over-relaxes the consensus step: xc is replaced by oalpha xc + (1 - oalpha) z_old in the
-// z- and mu-updates (Boyd et al. 3.4.3); the primal residual keeps the true xc.
-// fuse != 0: the last block to finish reduces the block partials in a fixed order and applies the control step.
-__global__ void __launch_bounds__(EDGE_THREADS, 6)
-edge_kernel(int nE, int nHown, const int *__restrict__ edge_he_tail, const int *__restrict__ edge_he_head,
-            const unsigned char *__restrict__ edge_counted, const double *__restrict__ xc, double *__restrict__ mu,
-            double *__restrict__ z, Ctrl *ctrl, double *__restrict__ partials, unsigned int *ticket, int fuse,
-            GcsParams p, long long n_x, long long n_mu, double *hist, int hist_cap, int nHghost, const PeerView *PVp, const double *__restrict__ tile_res, int ntiles) {
-    if (ctrl->stop && !ctrl->ignore_stop) return;
-    if (fuse == 2) peer_wait_halo(*PVp);
-    const double ms = ctrl->mu_scale, oa = p.outer_alpha, ob = 1.0 - p.outer_alpha;
-    // peer mode: the ghost slots of this iteration's parity (PVp lives in device memory: indexed at run time)
-    const int gpar = fuse == 2 ? ((PVp->comm[PVp->rank]->k + 1) & 1) * nHghost : 0;
-    double r2 = 0, dz2 = 0, x2 = 0, z2 = 0, m2 = 0;
-    // 40 registers per thread (6 blocks of 256 per SM), each thread with its index loads and then five independent data loads in flight
-    const unsigned n = 5u * (unsigned)nE, stride = gridDim.x * blockDim.x;
-    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const unsigned e = i / 5u, c = i - 5u * e;
-        const int ht = edge_he_tail[e], hh = edge_he_head[e];
-        const bool ot = ht < nHown, oh = hh < nHown;
-        const unsigned it_ = 5u * (unsigned)(ot ? ht : ht + gpar) + c, ih_ = 5u * (unsigned)(oh ? hh : hh + gpar) + c;
-        const double xt = xc[it_], xh = xc[ih_], zo = z[i];
-        const double mt = ot ? mu[it_] : 0.0, mh = oh ? mu[ih_] : 0.0;       // issued with the xc loads, not after the arithmetic
-        const double w = edge_counted ? (double)edge_counted[e] : 1.0;
-        double at = xt, ah = xh;
-        if (oa != 1.0) { at = oa * xt + ob * zo; ah = oa * xh + ob * zo; }
-        const double zn = 0.5 * (at + ah), dd = zn - zo;
-        z[i] = zn;
-        dz2 += w * dd * dd; z2 += w * zn * zn;
-        if (ot) { const double r = zn - xt, mn = ms * mt + (zn - at); mu[it_] = mn; r2 += r * r; x2 += xt * xt; m2 += mn * mn; }
-        if (oh) { const double r = zn - xh, mn = ms * mh + (zn - ah); mu[ih_] = mn; r2 += r * r; x2 += xh * xh; m2 += mn * mn; }
-    }
-    const double none = (blockIdx.x == 0 && threadIdx.x == 0) ? -1.0 : 0.0;      // global-coordinate residuals: this kernel works in global frames already
-    edge_finish(r2, dz2, x2, z2, m2, none, none, ctrl, partials, ticket, fuse, p, n_x, n_mu, hist, hist_cap, PVp, tile_res, ntiles);
-}
-
 // local frames (perf-mode option, vertex_perf.cuh GcsPerfTables.edge_delta): the consensus constraint of edge e is
 //   x_head = z,  x_tail = B z,  B (p1, p2, y) = (p1, p2 - y delta, y)
 // so the z-update is the least-squares solve  (I + B'B) z = x_head + B' x_tail  (the duals drop out: B' mu_tail + mu_head = 0 is an
 // invariant of the iteration), closed form per edge; mu_head += z - x_head, mu_tail += B z - x_tail; the dual residual is
-// rho sqrt(|dz|^2 + |B dz|^2).  One thread per edge: the three coupled scalars (p2, y) are needed together.
+// rho sqrt(|dz|^2 + |B dz|^2).  Global frames are delta = 0.  The three coupled scalars (p2, y) are needed together, so a thread
+// works on whole edges.
+// oalpha != 1 (perf mode only) over-relaxes the consensus step (Boyd et al. 3.4.3): x is replaced by oalpha x + (1 - oalpha) (B) z_old
+// in the z- and mu-updates; the primal residual keeps the true x.  B' mu_tail + mu_head = 0 stays invariant.
+// fuse != 0: the last block to finish reduces the block partials in a fixed order and applies the control step.
+// The two kernels below share the per-edge arithmetic through these helpers, so their z and mu agree bit for bit.
+
+// z-update of one edge: the relaxed copies at / ah of the tail's and head's points, the new z and its tail-side image B z
+template <bool OA>
+__device__ __forceinline__ void edge_z_update(const double (&xt)[5], const double (&xh)[5], const double (&zo)[5], double d0, double d1,
+                                              double oa, double ob, double (&at)[5], double (&ah)[5], double (&zn)[5], double (&bz)[5]) {
+#pragma unroll
+    for (int c = 0; c < 5; ++c) { at[c] = xt[c]; ah[c] = xh[c]; }
+    if (OA) {          // (compile-time: without over-relaxation at / ah are xt / xh and cost no registers)
+        const double bo[5] = {zo[0], zo[1], zo[2] - d0 * zo[4], zo[3] - d1 * zo[4], zo[4]};
+#pragma unroll
+        for (int c = 0; c < 5; ++c) { at[c] = oa * xt[c] + ob * bo[c]; ah[c] = oa * xh[c] + ob * zo[c]; }
+    }
+    zn[0] = 0.5 * (ah[0] + at[0]); zn[1] = 0.5 * (ah[1] + at[1]);
+    const double q0 = ah[2] + at[2], q1 = ah[3] + at[3], q2 = ah[4] + at[4] - (d0 * at[2] + d1 * at[3]);
+    zn[4] = (q2 + 0.5 * (d0 * q0 + d1 * q1)) / (2.0 + 0.5 * (d0 * d0 + d1 * d1));
+    zn[2] = 0.5 * (q0 + d0 * zn[4]); zn[3] = 0.5 * (q1 + d1 * zn[4]);
+    bz[0] = zn[0]; bz[1] = zn[1]; bz[2] = zn[2] - d0 * zn[4]; bz[3] = zn[3] - d1 * zn[4]; bz[4] = zn[4];
+}
+
+// |v|^2 + |B v|^2 of an edge vector v, its squared norm over both half-edge copies (the callers halve it); b2, b3: the two
+// scalars of B v that differ from v
+__device__ __forceinline__ double copies_sq(const double (&v)[5], double b2, double b3) {
+    return 2.0 * (v[0] * v[0] + v[1] * v[1] + v[4] * v[4]) + v[2] * v[2] + v[3] * v[3] + b2 * b2 + b3 * b3;
+}
+
+// dual update of one half-edge with copy p of the edge's point (B z on the tail side, z on the head side), primal copy x and relaxed
+// copy a: out[off + c] <- ms * mu + (p - a); with acc, adds |p - x|^2, |x|^2, |mu_new|^2, scalar by scalar.  (A base and an offset,
+// not one pointer: with a pointer the warp-cooperative kernel's shared-memory addressing takes more instructions.)
+__device__ __forceinline__ void half_edge_dual(const double (&p)[5], const double (&x)[5], const double (&a)[5], const double (&mu)[5], double ms,
+                                               double *out, size_t off, bool acc, double &r2, double &x2, double &m2) {
+#pragma unroll
+    for (int c = 0; c < 5; ++c) {
+        const double r = p[c] - x[c], mn = ms * mu[c] + (p[c] - a[c]);
+        out[off + c] = mn;
+        if (acc) { r2 += r * r; x2 += x[c] * x[c]; m2 += mn * mn; }
+    }
+}
+
+// One thread per edge: partitions with ghost slots (multi-GPU), edge_counted weights, the check variant.
 // GRES (check variant, local frames only): also the primal / dual residual sums in GLOBAL coordinates.  The copies of an edge
 // (u, w) live in the frame of u (both points of the tail's copy, the first point of the head's copy) or of w (the head's own first
 // point); adding  flow * centre-of-frame  to a point gives its global value, so  r_global = r_local + r_flow * centre.
-template <int MINB, bool OA, bool GRES>
-__global__ void __launch_bounds__(EDGE_THREADS, MINB)
+// 128 registers (2 resident blocks per SM): all 25 loads of an edge are in flight together.
+template <bool OA, bool GRES>
+__global__ void __launch_bounds__(EDGE_THREADS, 2)
 edge_frames_kernel(int nE, int nHown, const int *__restrict__ edge_he_tail, const int *__restrict__ edge_he_head,
                    const unsigned char *__restrict__ edge_counted, const double *__restrict__ edge_delta, const double *__restrict__ edge_cent, const double *__restrict__ xc,
                    double *__restrict__ mu, double *__restrict__ z, Ctrl *ctrl, double *__restrict__ partials, unsigned int *ticket, int fuse,
@@ -401,6 +409,7 @@ edge_frames_kernel(int nE, int nHown, const int *__restrict__ edge_he_tail, cons
     if (ctrl->stop && !ctrl->ignore_stop) return;
     if (fuse == 2) peer_wait_halo(*PVp);
     const double ms = ctrl->mu_scale, oa = p.outer_alpha, ob = 1.0 - p.outer_alpha;
+    // peer mode: the ghost slots of this iteration's parity (PVp lives in device memory: indexed at run time)
     const int gpar = fuse == 2 ? ((PVp->comm[PVp->rank]->k + 1) & 1) * nHghost : 0;
     double r2 = 0, dz2 = 0, x2 = 0, z2 = 0, m2 = 0, r2g = 0, dz2g = 0;
     if (!GRES && blockIdx.x == 0 && threadIdx.x == 0) r2g = dz2g = -1.0;      // "not computed in this iteration"
@@ -417,61 +426,32 @@ edge_frames_kernel(int nE, int nHown, const int *__restrict__ edge_he_tail, cons
         double xt[5], xh[5], zo[5], mt[5], mh[5];
 #pragma unroll
         for (int c = 0; c < 5; ++c) { xt[c] = pt[c]; xh[c] = ph[c]; zo[c] = z[5 * (size_t)e + c]; }
-        // MINB == 2 (128 registers): the duals are loaded together with the copies (maximum memory-level parallelism per thread);
-        // MINB > 2 (<= 80 / 64 registers, more resident warps): they are loaded after z has been written, one side at a time
-        if (MINB == 2) {
 #pragma unroll
-            for (int c = 0; c < 5; ++c) { mt[c] = ot ? mu[5 * (size_t)ht_ + c] : 0.0; mh[c] = oh ? mu[5 * (size_t)hh_ + c] : 0.0; }
-        }
+        for (int c = 0; c < 5; ++c) { mt[c] = ot ? mu[5 * (size_t)ht_ + c] : 0.0; mh[c] = oh ? mu[5 * (size_t)hh_ + c] : 0.0; }
         const double d0 = edge_delta ? edge_delta[2 * (size_t)e] : 0.0, d1 = edge_delta ? edge_delta[2 * (size_t)e + 1] : 0.0;
         const double w = edge_counted ? (double)edge_counted[e] : 1.0;
-        double zn[5], bz[5], at[5], ah[5];
-        // oalpha != 1: over-relaxed consensus step (Boyd et al. 3.4.3) — x is replaced by oalpha x + (1 - oalpha) (B) z_old in the z- and
-        // mu-updates; the primal residual keeps the true x.  B' mu_tail + mu_head = 0 stays invariant.
-#pragma unroll
-        for (int c = 0; c < 5; ++c) { at[c] = xt[c]; ah[c] = xh[c]; }
-        if (OA) {          // (compile-time: without over-relaxation at / ah are xt / xh and cost no registers)
-            const double bo[5] = {zo[0], zo[1], zo[2] - d0 * zo[4], zo[3] - d1 * zo[4], zo[4]};
-#pragma unroll
-            for (int c = 0; c < 5; ++c) { at[c] = oa * xt[c] + ob * bo[c]; ah[c] = oa * xh[c] + ob * zo[c]; }
-        }
-        zn[0] = 0.5 * (ah[0] + at[0]); zn[1] = 0.5 * (ah[1] + at[1]);
-        const double q0 = ah[2] + at[2], q1 = ah[3] + at[3], q2 = ah[4] + at[4] - (d0 * at[2] + d1 * at[3]);
-        zn[4] = (q2 + 0.5 * (d0 * q0 + d1 * q1)) / (2.0 + 0.5 * (d0 * d0 + d1 * d1));
-        zn[2] = 0.5 * (q0 + d0 * zn[4]); zn[3] = 0.5 * (q1 + d1 * zn[4]);
-        bz[0] = zn[0]; bz[1] = zn[1]; bz[2] = zn[2] - d0 * zn[4]; bz[3] = zn[3] - d1 * zn[4]; bz[4] = zn[4];
-        double dd[5];
+        double at[5], ah[5], zn[5], bz[5], dd[5];
+        edge_z_update<OA>(xt, xh, zo, d0, d1, oa, ob, at, ah, zn, bz);
 #pragma unroll
         for (int c = 0; c < 5; ++c) { dd[c] = zn[c] - zo[c]; z[5 * (size_t)e + c] = zn[c]; }
         const double db2 = dd[2] - d0 * dd[4], db3 = dd[3] - d1 * dd[4];
-        dz2 += 0.5 * w * (2.0 * (dd[0] * dd[0] + dd[1] * dd[1] + dd[4] * dd[4]) + dd[2] * dd[2] + dd[3] * dd[3] + db2 * db2 + db3 * db3);
-        z2 += 0.5 * w * (2.0 * (zn[0] * zn[0] + zn[1] * zn[1] + zn[4] * zn[4]) + zn[2] * zn[2] + zn[3] * zn[3] + bz[2] * bz[2] + bz[3] * bz[3]);
+        dz2 += 0.5 * w * copies_sq(dd, db2, db3);
+        z2 += 0.5 * w * copies_sq(zn, bz[2], bz[3]);
         double cu0 = 0.0, cu1 = 0.0, cw0 = 0.0, cw1 = 0.0;
         if (GRES) {
             cu0 = edge_cent[2 * (size_t)e]; cu1 = edge_cent[2 * (size_t)e + 1]; cw0 = cu0 - d0; cw1 = cu1 - d1;
             const double g0 = dd[0] + dd[4] * cu0, g1 = dd[1] + dd[4] * cu1, g2 = dd[2] + dd[4] * cw0, g3 = dd[3] + dd[4] * cw1;
             dz2g += w * (g0 * g0 + g1 * g1 + g2 * g2 + g3 * g3 + dd[4] * dd[4]);
         }
-        if (MINB > 2) asm volatile("" ::: "memory");     // keeps the compiler from hoisting the dual loads above this point
         if (ot) {
-            if (MINB > 2) {
-#pragma unroll
-                for (int c = 0; c < 5; ++c) mt[c] = mu[5 * (size_t)ht_ + c];
-            }
-#pragma unroll
-            for (int c = 0; c < 5; ++c) { const double r = bz[c] - xt[c], mn = ms * mt[c] + (bz[c] - at[c]); mu[5 * (size_t)ht_ + c] = mn; r2 += r * r; x2 += xt[c] * xt[c]; m2 += mn * mn; }
+            half_edge_dual(bz, xt, at, mt, ms, mu, 5 * (size_t)ht_, true, r2, x2, m2);
             if (GRES) {      // every slot of the tail's copy lives in the tail's frame
                 const double ry = bz[4] - xt[4], a0 = bz[0] - xt[0] + ry * cu0, a1 = bz[1] - xt[1] + ry * cu1, a2 = bz[2] - xt[2] + ry * cu0, a3 = bz[3] - xt[3] + ry * cu1;
                 r2g += a0 * a0 + a1 * a1 + a2 * a2 + a3 * a3 + ry * ry;
             }
         }
         if (oh) {
-            if (MINB > 2) {
-#pragma unroll
-                for (int c = 0; c < 5; ++c) mh[c] = mu[5 * (size_t)hh_ + c];
-            }
-#pragma unroll
-            for (int c = 0; c < 5; ++c) { const double r = zn[c] - xh[c], mn = ms * mh[c] + (zn[c] - ah[c]); mu[5 * (size_t)hh_ + c] = mn; r2 += r * r; x2 += xh[c] * xh[c]; m2 += mn * mn; }
+            half_edge_dual(zn, xh, ah, mh, ms, mu, 5 * (size_t)hh_, true, r2, x2, m2);
             if (GRES) {      // the tail's first point in the tail's frame, the head's own first point in the head's frame
                 const double ry = zn[4] - xh[4], a0 = zn[0] - xh[0] + ry * cu0, a1 = zn[1] - xh[1] + ry * cu1, a2 = zn[2] - xh[2] + ry * cw0, a3 = zn[3] - xh[3] + ry * cw1;
                 r2g += a0 * a0 + a1 * a1 + a2 * a2 + a3 * a3 + ry * ry;
@@ -487,11 +467,10 @@ edge_frames_kernel(int nE, int nHown, const int *__restrict__ edge_he_tail, cons
 // pass k handles double l + 32 k, i.e. scalar (l + 32 k) % 5 of record (l + 32 k) / 5, the record's index coming from the lane that
 // owns the edge by a shuffle) — a request then touches ~7 records instead of 32, a third of the L1 wavefronts of the
 // one-thread-per-record pattern; each lane then reads / writes its own edge's records in shared memory with stride 5 (conflict-free).
-// The arithmetic per edge is the one of edge_frames_kernel, expression by expression (bit-identical z and mu).
 #define COOP_WARPS (EDGE_THREADS / 32)
 #define COOP_SMEM_DOUBLES (COOP_WARPS * 5 * 160)
-template <bool OA, int MINB>
-__global__ void __launch_bounds__(EDGE_THREADS, MINB)
+template <bool OA>
+__global__ void __launch_bounds__(EDGE_THREADS, 2)
 edge_coop_kernel(int nE, const int *__restrict__ edge_he_tail, const int *__restrict__ edge_he_head, const double *__restrict__ edge_delta,
                  const double *__restrict__ xc, double *__restrict__ mu, double *__restrict__ z, Ctrl *ctrl, double *__restrict__ partials,
                  unsigned int *ticket, int fuse, GcsParams p, long long n_x, long long n_mu, double *hist, int hist_cap,
@@ -536,39 +515,19 @@ edge_coop_kernel(int nE, const int *__restrict__ edge_he_tail, const int *__rest
 #pragma unroll
         for (int c = 0; c < 5; ++c) { xt[c] = xtS[5 * lane + c]; xh[c] = xhS[5 * lane + c]; zo[c] = zoS[5 * lane + c]; mt[c] = mtS[5 * lane + c]; mh[c] = mhS[5 * lane + c]; }
         __syncwarp();                    // every lane has read its records: the buffers can take the results
-        double zn[5], bz[5], at[5], ah[5];
-#pragma unroll
-        for (int c = 0; c < 5; ++c) { at[c] = xt[c]; ah[c] = xh[c]; }
-        if (OA) {
-            const double bo[5] = {zo[0], zo[1], zo[2] - d0 * zo[4], zo[3] - d1 * zo[4], zo[4]};
-#pragma unroll
-            for (int c = 0; c < 5; ++c) { at[c] = oa * xt[c] + ob * bo[c]; ah[c] = oa * xh[c] + ob * zo[c]; }
-        }
-        zn[0] = 0.5 * (ah[0] + at[0]); zn[1] = 0.5 * (ah[1] + at[1]);
-        const double q0 = ah[2] + at[2], q1 = ah[3] + at[3], q2 = ah[4] + at[4] - (d0 * at[2] + d1 * at[3]);
-        zn[4] = (q2 + 0.5 * (d0 * q0 + d1 * q1)) / (2.0 + 0.5 * (d0 * d0 + d1 * d1));
-        zn[2] = 0.5 * (q0 + d0 * zn[4]); zn[3] = 0.5 * (q1 + d1 * zn[4]);
-        bz[0] = zn[0]; bz[1] = zn[1]; bz[2] = zn[2] - d0 * zn[4]; bz[3] = zn[3] - d1 * zn[4]; bz[4] = zn[4];
-        double dd[5];
+        double at[5], ah[5], zn[5], bz[5], dd[5];
+        edge_z_update<OA>(xt, xh, zo, d0, d1, oa, ob, at, ah, zn, bz);
 #pragma unroll
         for (int c = 0; c < 5; ++c) { dd[c] = zn[c] - zo[c]; zoS[5 * lane + c] = zn[c]; }
+        // (db2 / db3 stay outside the branch: ptxas fuses a multiply and an add into one FMA only inside one block, so where they
+        // are computed decides the last bits of dz2)
         const double db2 = dd[2] - d0 * dd[4], db3 = dd[3] - d1 * dd[4];
         if (valid) {
-            dz2 += 0.5 * (2.0 * (dd[0] * dd[0] + dd[1] * dd[1] + dd[4] * dd[4]) + dd[2] * dd[2] + dd[3] * dd[3] + db2 * db2 + db3 * db3);
-            z2 += 0.5 * (2.0 * (zn[0] * zn[0] + zn[1] * zn[1] + zn[4] * zn[4]) + zn[2] * zn[2] + zn[3] * zn[3] + bz[2] * bz[2] + bz[3] * bz[3]);
+            dz2 += 0.5 * copies_sq(dd, db2, db3);
+            z2 += 0.5 * copies_sq(zn, bz[2], bz[3]);
         }
-#pragma unroll
-        for (int c = 0; c < 5; ++c) {
-            const double r = bz[c] - xt[c], mn = ms * mt[c] + (bz[c] - at[c]);
-            mtS[5 * lane + c] = mn;
-            if (valid) { r2 += r * r; x2 += xt[c] * xt[c]; m2 += mn * mn; }
-        }
-#pragma unroll
-        for (int c = 0; c < 5; ++c) {
-            const double r = zn[c] - xh[c], mn = ms * mh[c] + (zn[c] - ah[c]);
-            mhS[5 * lane + c] = mn;
-            if (valid) { r2 += r * r; x2 += xh[c] * xh[c]; m2 += mn * mn; }
-        }
+        half_edge_dual(bz, xt, at, mt, ms, mtS, 5 * lane, valid, r2, x2, m2);
+        half_edge_dual(zn, xh, ah, mh, ms, mhS, 5 * lane, valid, r2, x2, m2);
         __syncwarp();
         // ---- shared memory -> HBM, the same five passes
 #pragma unroll
@@ -805,26 +764,20 @@ static int create_impl(GcsHandle *h, const GcsGraph *g) {
     CK(cudaFuncSetAttribute(vertex_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, h->k1_smem));
     CK(cudaFuncSetAttribute(vertex_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     h->k1_blocks = (g->nV + h->k1_warps - 1) / h->k1_warps;
-    {   // edge kernel: 5 threads per edge, a whole number of waves of resident blocks (8 blocks of 256 threads per SM)
-        const long long need = (5ll * g->nE + EDGE_THREADS - 1) / EDGE_THREADS;
-        // measured on the 100k-vertex grid: warp-cooperative 38 us (2 blocks per SM; 44 us with 3), one thread per edge 54 us,
-        // one thread per (edge, scalar) 68 us (6 blocks per SM) .. 84 us (24); the env variables are tuning knobs
-        const char *bps = getenv("GCS_EDGE_BLOCKS_PER_SM"), *ek = getenv("GCS_EDGE_KERNEL");
-        h->edge_per_edge = !(ek && !strcmp(ek, "per_scalar"));
-        // warp-cooperative variant: the default wherever it applies (single GPU, no ghost slots, throughput path): 38 us vs 54 us
-        // for one thread per edge on the 100k-vertex grid; GCS_EDGE_KERNEL=per_edge / per_scalar select the others
-        h->edge_coop = !(ek && (!strcmp(ek, "per_edge") || !strcmp(ek, "per_scalar")));
-        h->coop_blocks = prop.multiProcessorCount * (bps && atoi(bps) > 0 ? atoi(bps) : 2);
-        const char *mb = getenv("GCS_EDGE_MINB");        // register budget of the per-edge kernel: 2, 3 or 4 resident blocks per SM
-        h->edge_minb = mb && atoi(mb) >= 2 && atoi(mb) <= 4 ? atoi(mb) : 2;
+    {   // edge kernels.  Measured on the 100k-vertex grid: warp-cooperative 38 us (2 blocks per SM; 44 us with 3), one thread per
+        // edge 54 us (2 blocks per SM).  The warp-cooperative kernel runs wherever it applies (single GPU, no ghost slots,
+        // throughput path).  GCS_EDGE_KERNEL=per_edge runs the one-thread-per-edge kernel there too: this is how a test runs both
+        // kernels on one state, which must agree bit for bit.
+        const char *ek = getenv("GCS_EDGE_KERNEL");
+        h->edge_coop = !(ek && !strcmp(ek, "per_edge"));
+        h->coop_blocks = 2 * prop.multiProcessorCount;
         if (h->edge_coop) {
             const int smb = (int)(sizeof(double) * COOP_SMEM_DOUBLES);
-            CK(cudaFuncSetAttribute(edge_coop_kernel<false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smb));
-            CK(cudaFuncSetAttribute(edge_coop_kernel<true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smb));
-            CK(cudaFuncSetAttribute(edge_coop_kernel<false, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smb));
-            CK(cudaFuncSetAttribute(edge_coop_kernel<true, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smb));
+            CK(cudaFuncSetAttribute(edge_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smb));
+            CK(cudaFuncSetAttribute(edge_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smb));
         }
-        const long long cap = (long long)prop.multiProcessorCount * (bps && atoi(bps) > 0 ? atoi(bps) : (h->edge_per_edge ? 4 : 6));
+        // one thread per edge, at most 4 blocks per SM; at least as many blocks as the warp-cooperative launch (partials rows)
+        const long long need = (g->nE + EDGE_THREADS - 1) / EDGE_THREADS, cap = 4ll * prop.multiProcessorCount;
         h->edge_blocks = (int)(need < 1 ? 1 : (need > cap ? cap : need));
     }
     CK(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
@@ -946,35 +899,23 @@ static int launch_edge(GcsHandle *h, int fuse) {
                                                                      h->ctrl, h->p, h->prob_nx, h->prob_nmu, h->hist, h->hist_cap);
         return 0;
     }
+    const bool oa = h->p.outer_alpha != 1.0;
     if (h->edge_coop && h->nHghost == 0 && !h->edge_counted && !(h->perf_on && h->inner_on)) {     // single-GPU throughput path
         const int nchunks = (h->nE + 31) / 32;
         int blocks = (nchunks + COOP_WARPS - 1) / COOP_WARPS;
         if (blocks > h->coop_blocks) blocks = h->coop_blocks;
         if (blocks < 1) blocks = 1;
-        const size_t sm = sizeof(double) * COOP_SMEM_DOUBLES;
-#define EDGE_COOP(OA, MINB) edge_coop_kernel<OA, MINB><<<blocks, EDGE_THREADS, sm, h->stream>>>(h->nE, h->edge_he_tail, h->edge_he_head, h->perf_on ? h->p_edge_delta : nullptr, \
-            h->xc, h->mu, h->z, h->ctrl, h->partials, h->ticket, fuse, h->p, h->n_x, h->n_mu, h->hist, h->hist_cap, INNER_ARGS(h))
-        if (h->p.outer_alpha != 1.0) { if (h->edge_minb >= 3) EDGE_COOP(true, 3); else EDGE_COOP(true, 2); }
-        else { if (h->edge_minb >= 3) EDGE_COOP(false, 3); else EDGE_COOP(false, 2); }
-#undef EDGE_COOP
+        auto *k = oa ? edge_coop_kernel<true> : edge_coop_kernel<false>;
+        k<<<blocks, EDGE_THREADS, sizeof(double) * COOP_SMEM_DOUBLES, h->stream>>>(h->nE, h->edge_he_tail, h->edge_he_head, h->perf_on ? h->p_edge_delta : nullptr,
+            h->xc, h->mu, h->z, h->ctrl, h->partials, h->ticket, fuse, h->p, h->n_x, h->n_mu, h->hist, h->hist_cap, INNER_ARGS(h));
         return 0;
     }
-    if ((h->perf_on && h->p_edge_delta) || h->edge_per_edge) {      // local frames (or the one-thread-per-edge variant by request)
-        int blocks = (h->nE + EDGE_THREADS - 1) / EDGE_THREADS;
-        if (blocks > h->edge_blocks) blocks = h->edge_blocks;
-        if (blocks < 1) blocks = 1;
-        const bool gres = h->perf_on && h->inner_on && h->p_edge_delta && h->p_edge_cent;      // check variant in local frames
-#define EDGE_FRAMES(MINB) if (gres) { if (h->p.outer_alpha != 1.0) EDGE_FRAMES_(MINB, true, true); else EDGE_FRAMES_(MINB, false, true); } \
-                          else { if (h->p.outer_alpha != 1.0) EDGE_FRAMES_(MINB, true, false); else EDGE_FRAMES_(MINB, false, false); }
-#define EDGE_FRAMES_(MINB, OA, GRES) edge_frames_kernel<MINB, OA, GRES><<<blocks, EDGE_THREADS, 0, h->stream>>>(h->nE, h->nHown, h->edge_he_tail, h->edge_he_head, h->edge_counted, \
-            h->perf_on ? h->p_edge_delta : nullptr, h->perf_on ? h->p_edge_cent : nullptr, h->xc, h->mu, h->z, h->ctrl, h->partials, h->ticket, fuse, h->p, h->n_x, h->n_mu, h->hist, h->hist_cap, h->nHghost, h->PV_dev, INNER_ARGS(h))
-        if (h->edge_minb == 4) { EDGE_FRAMES(4); } else if (h->edge_minb == 3) { EDGE_FRAMES(3); } else { EDGE_FRAMES(2); }
-#undef EDGE_FRAMES
-#undef EDGE_FRAMES_
-        return 0;
-    }
-    edge_kernel<<<h->edge_blocks, EDGE_THREADS, 0, h->stream>>>(h->nE, h->nHown, h->edge_he_tail, h->edge_he_head, h->edge_counted, h->xc, h->mu, h->z, h->ctrl,
-                                                                h->partials, h->ticket, fuse, h->p, h->n_x, h->n_mu, h->hist, h->hist_cap, h->nHghost, h->PV_dev, INNER_ARGS(h));
+    const bool gres = h->perf_on && h->inner_on && h->p_edge_delta && h->p_edge_cent;      // check variant in local frames
+    auto *k = gres ? (oa ? edge_frames_kernel<true, true> : edge_frames_kernel<false, true>)
+                   : (oa ? edge_frames_kernel<true, false> : edge_frames_kernel<false, false>);
+    k<<<h->edge_blocks, EDGE_THREADS, 0, h->stream>>>(h->nE, h->nHown, h->edge_he_tail, h->edge_he_head, h->edge_counted,
+        h->perf_on ? h->p_edge_delta : nullptr, h->perf_on ? h->p_edge_cent : nullptr, h->xc, h->mu, h->z, h->ctrl, h->partials, h->ticket, fuse, h->p,
+        h->n_x, h->n_mu, h->hist, h->hist_cap, h->nHghost, h->PV_dev, INNER_ARGS(h));
     return 0;
 }
 static int launch_ctrl(GcsHandle *h) {

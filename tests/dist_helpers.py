@@ -1,6 +1,6 @@
 """CPU stand-in for the CUDA backend of ``gcs_admm_b200.dist.DistributedADMM`` (tests only):
 the x-update is the C oracle's, the edge/dual/residual/control arithmetic is restated in numpy with the
-same formulas as the kernels (csrc/gcsadmm.cu edge_kernel / control_kernel)."""
+same formulas as the kernels (csrc/gcsadmm.cu edge_frames_kernel in global frames / control_kernel)."""
 import ctypes as C
 
 import numpy as np
