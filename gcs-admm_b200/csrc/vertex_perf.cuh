@@ -20,7 +20,7 @@
 //
 // Mapping: a thread block works on one TILE of consecutive vertices at a time (<= 64 blocks = 256 pairs; the kernel's blocks are
 // persistent and walk tiles, staging the next one while they compute — gcsadmm.cu vertex_perf_kernel); every phase is a flat loop
-// over (pair | block variable | vertex) items of the whole tile, so lanes stay busy whatever the degrees are; phases
+// over (half-edge point | block variable | vertex) items of the whole tile, so lanes stay busy whatever the degrees are; phases
 // exchange data through shared memory only.  The per-tile state t, the cone records and the path-length state are
 // contiguous in HBM and move with 1-D bulk async copies (cp.async.bulk + mbarrier).
 //
@@ -319,6 +319,16 @@ GCS_DEV void gcs_cstep_store(double *t, double *e, double t0, double t1, double 
     t[0] = q0 - l0; t[1] = q1 - l1; t[2] = q2 - l2;
     e[0] = (1.0 - alpha) * q0 + l0; e[1] = (1.0 - alpha) * q1 + l1; e[2] = (1.0 - alpha) * q2 + l2;
 }
+// t-step of one pair p = M u + m0:  t = alpha p + e.  INNER, last pass: also adds the pair's squared inner residual |p - c|^2 to
+// rin (t holds d = c - lam, e = (1 - alpha) c + lam  =>  c = (d + e) / (2 - alpha))
+template <bool INNER>
+GCS_DEV void gcs_tstep(double *t, const double *e, double p0, double p1, double p2, double alpha, bool last, double &rin) {
+    if (INNER && last) {
+        const double ic = 1.0 / (2.0 - alpha), r0 = p0 - ic * (t[0] + e[0]), r1 = p1 - ic * (t[1] + e[1]), r2 = p2 - ic * (t[2] + e[2]);
+        rin += r0 * r0 + r1 * r1 + r2 * r2;
+    }
+    t[0] = alpha * p0 + e[0]; t[1] = alpha * p1 + e[1]; t[2] = alpha * p2 + e[2];
+}
 
 // x-update of one tile of vertices in perf mode.  S: work arrays, B: the tile's staged arrays (device build: already filled by
 // gcs_perf_stage and waited for; the new state leaves B by bulk stores of GCS_COPY_THREAD).  Device build: after the tile's first
@@ -365,7 +375,7 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
 #endif
     // Until the first barrier of a pass the block works as two groups: the first half of the warps does the c-step, two pairs per
     // thread; the others issue the gathers of the consensus targets, answer the forced-zero half-edges and do the path-length item
-    // meanwhile.  A one-warp block does both, one after the other.
+    // meanwhile.  After the v-step the same two groups split the t-step (P7).  A one-warp block does both, one after the other.
 #if defined(GCS_EMULATE)
     const bool cgrp = true, ggrp = true;
     const int cid = 0, cn = 1, gid0 = 0, gn = 1;
@@ -509,34 +519,49 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
         }
 #endif
         GCS_CTA_SYNC();
-        // ---- P7: block variables  u = dinv r + beta  (evaluated where they are used), t-step  t = alpha (M u + m0) + e;  on the
-        // last pass the vertex outputs and the consensus copies xc in edge-canonical order (:492-522)
-        GCS_CTA_LOOP(p, 4 * nb) {
-            const int b = p >> 2, i = (p >> 1) & 1, fam = p & 1, info = binfo(b), vl = info & 255;
+        // ---- P7: block variables  u = dinv r + beta,  t-step  t = alpha (M u + m0) + e;  on the last pass the vertex outputs and the
+        // consensus copies xc in edge-canonical order (:492-522).  Split like P1 / P2: the first half of the warps takes the half-edge
+        // points, the others the path-length item and the vertex outputs, which read only cout, tnS and enS.
+        // Item j = point i of block b (j = 2 b + i): u(b, 2 i), u(b, 2 i + 1) and the flow u(b, 4) are evaluated once for both pairs
+        // of the point, and on the last pass they are also the point's share of xc
+        if (cgrp) for (int j = cid; j < 2 * nb; j += cn) {
+            const int b = j >> 1, i = j & 1, info = binfo(b), vl = info & 255;
             const int *w = vi + GCS_VI_N * vl;
-            if (!ACT_W || ((info >> 10) & fam)) continue;
-            const double *co = cout + GCS_NCX * vl, *tab = T.cls_tab + (size_t)GCS_CLS_STRIDE * w[GCS_VI_CLS], *e = eS + 3 * p;
-            double p0 = gcs_block_u(rS, co, tab, info, b, 2 * i), p1 = gcs_block_u(rS, co, tab, info, b, 2 * i + 1), p2 = gcs_block_u(rS, co, tab, info, b, 4);
-            if (fam) { p0 = co[2 * i] - p0; p1 = co[2 * i + 1] - p1; p2 = 1.0 - p2; }
-            double *t = tS + 3 * p;
-            if (INNER && last) {      // inner residual  (M u + m0) - c  of the pair:  t holds d = c - lam, e = (1 - alpha) c + lam  =>  c = (d + e) / (2 - alpha)
-                const double ic = 1.0 / (2.0 - alpha), r0 = p0 - ic * (t[0] + e[0]), r1 = p1 - ic * (t[1] + e[1]), r2_ = p2 - ic * (t[2] + e[2]);
-                rin += r0 * r0 + r1 * r1 + r2_ * r2_;
+            if (!ACT_W) continue;
+            const double *co = cout + GCS_NCX * vl, *tab = T.cls_tab + (size_t)GCS_CLS_STRIDE * w[GCS_VI_CLS], *e = eS + 6 * j;
+            const double u0 = gcs_block_u(rS, co, tab, info, b, 2 * i), u1 = gcs_block_u(rS, co, tab, info, b, 2 * i + 1), u4 = gcs_block_u(rS, co, tab, info, b, 4);
+            double *t = tS + 6 * j;
+            gcs_tstep<INNER>(t, e, u0, u1, u4, alpha, last, rin);                                     // fam 0: (a_i, y_e)
+            if (!((info >> 10) & 1)) gcs_tstep<INNER>(t + 3, e + 3, co[2 * i] - u0, co[2 * i + 1] - u1, 1.0 - u4, alpha, last, rin);   // fam 1: (x_i - a_i, 1 - y_e)
+            const int h = bhe(b);
+            if (last && h >= 0) {
+                // out-edge: point i is slots 2 i, 2 i + 1 (own first point | other's first point == own second point, C5);
+                // in-edge: point 0 is slots 2, 3 (own first point), slots 0, 1 are the other copy's free first point -> its target
+                const bool out = (info >> 8) & 1;
+                double *x = St.xc + 5 * (size_t)h;
+                if (out || !i) { const int s = out ? 2 * i : 2; x[s] = u0; x[s + 1] = u1; }
+                else { x[0] = TS[5 * b]; x[1] = TS[5 * b + 1]; }
+                if (!i) x[4] = u4;
             }
-            t[0] = alpha * p0 + e[0]; t[1] = alpha * p1 + e[1]; t[2] = alpha * p2 + e[2];
         }
-        GCS_CTA_LOOP(i, nvt) {
-            const int *w = vi + GCS_VI_N * i;
-            if (!ACT_W || !w[GCS_VI_NB]) continue;
-            const double *zz = cout + GCS_NCX * i + 4;
-            if (INNER && last) {
-                const double ic = 1.0 / (2.0 - alpha), r0 = (zz[0] - zz[2]) - ic * (tnS[2 * i] + enS[2 * i]), r1 = (zz[1] - zz[3]) - ic * (tnS[2 * i + 1] + enS[2 * i + 1]);
-                rin += r0 * r0 + r1 * r1;
+        if (ggrp) {
+#if defined(GCS_EMULATE)
+            const int gid = gid0;
+#else
+            int gid = gid0;            // opaque, as in P1
+            asm volatile("" : "+r"(gid));
+#endif
+            for (int i = gid; i < nvt; i += gn) {
+                const int *w = vi + GCS_VI_N * i;
+                if (!ACT_W || !w[GCS_VI_NB]) continue;
+                const double *zz = cout + GCS_NCX * i + 4;
+                if (INNER && last) {
+                    const double ic = 1.0 / (2.0 - alpha), r0 = (zz[0] - zz[2]) - ic * (tnS[2 * i] + enS[2 * i]), r1 = (zz[1] - zz[3]) - ic * (tnS[2 * i + 1] + enS[2 * i + 1]);
+                    rin += r0 * r0 + r1 * r1;
+                }
+                tnS[2 * i] = alpha * (zz[0] - zz[2]) + enS[2 * i]; tnS[2 * i + 1] = alpha * (zz[1] - zz[3]) + enS[2 * i + 1];
             }
-            tnS[2 * i] = alpha * (zz[0] - zz[2]) + enS[2 * i]; tnS[2 * i + 1] = alpha * (zz[1] - zz[3]) + enS[2 * i + 1];
-        }
-        if (last) {
-            GCS_CTA_LOOP(q, 9 * nvt) {
+            if (last) for (int q = gid; q < 9 * nvt; q += gn) {
                 const int vl = q / 9, k = q - 9 * vl;
                 const int *w = vi + GCS_VI_N * vl;
                 if (!ACT_W || !w[GCS_VI_NB]) continue;
@@ -545,16 +570,6 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
                 if (T.edge_delta && k < 8)          // local frames: back to global coordinates  x = x' + c_v,  z_v = z_v' + y_v c_v
                     val += (k < 4 ? 1.0 : cout[GCS_NCX * vl + 8]) * G.cent[2 * v + (k & 1)];
                 if (k < 4) St.x_v[4 * v + k] = val; else if (k < 8) St.z_v[4 * v + k - 4] = val; else St.y_v[v] = val;
-            }
-            GCS_CTA_LOOP(q, 5 * nb) {
-                const int b = q / 5, c = q - 5 * b, h = bhe(b), info = binfo(b), vl = info & 255;
-                const int *w = vi + GCS_VI_N * vl;
-                if (h < 0 || !ACT_W) continue;
-                const double *co = cout + GCS_NCX * vl, *tab = T.cls_tab + (size_t)GCS_CLS_STRIDE * w[GCS_VI_CLS];
-                double x;
-                if ((info >> 8) & 1) x = gcs_block_u(rS, co, tab, info, b, c);      // out-edge: own first point | other's first point == own second point (C5)
-                else x = c < 2 ? TS[q] : gcs_block_u(rS, co, tab, info, b, c < 4 ? c - 2 : 4);   // in-edge: other's first point is free -> its target | own first point
-                St.xc[5 * (size_t)h + c] = x;
             }
         }
         if (!last) GCS_CTA_SYNC();     // (after the last pass P8's barrier follows)
