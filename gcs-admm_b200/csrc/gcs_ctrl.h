@@ -10,6 +10,8 @@ struct Ctrl {
     double pri_g, dual_g;   // local frames: the residuals in global coordinates (the reference's definition :598 / :602); -1: not computed
     double inner;       // perf mode: |(M u + m0) - c| over all (point, flow) pairs — how far the vertex programs' own constraints are from being met
     double sums[NSUMS];
+    double abs_tol;         // this problem's tolerance of the absolute stop rule (0: GcsParams.abs_tol)
     unsigned long long inner_iters, skipped;
     int it, stop, opt, diverged, inner_fail, ignore_stop;
+    int inner_active;       // batched perf mode: this problem is near its tolerance, the edge kernel adds up its inner residual (set by gcsadmm_run)
 };

@@ -94,7 +94,7 @@ struct GcsHandle {
     int *poly_off, *he_off, *he_edge, *edge_he_tail, *edge_he_head;
     double *polyA, *polyb, *cent;
     unsigned char *he_flags, *vtype, *edge_counted;
-    int *vprob, *prob_eoff; long long *prob_nx, *prob_nmu;   // batched mode (nP > 1)
+    int *vprob, *prob_voff, *prob_eoff; long long *prob_nx, *prob_nmu;   // batched mode (nP > 1)
     int *he_prob_host;  // host: problem of each half-edge (batched mode)
     unsigned int *ticket;   // edge kernels: blocks finished in the current launch (the last one reduces + controls)
     unsigned int *push_ticket;   // perf K1 in peer mode: blocks finished (the last one pushes the halo)
@@ -114,6 +114,7 @@ struct GcsHandle {
     GcsPerfTables PT;
     long long perf_nblocks;
     int *p_vclass, *p_cone_off, *p_blk_off, *p_blk_rec, *p_vrec, *p_tile_rec; double *p_cls_tab, *p_cone, *p_tstate, *p_tn, *p_edge_delta, *p_edge_cent, *p_tile_res;
+    double *p_pt_res, *p_vt_res;     // batched perf mode: the inner residual per item (GcsPerfTables.pt_res / vt_res)
     // one CUDA graph per chunk of `check_every` iterations (own stream only)
     cudaGraphExec_t graph_exec; int graph_iters;
     // peer mode (multi-GPU over NVLink peer memory, one process per GPU): see the "peer mode" section
@@ -205,7 +206,7 @@ vertex_perf_kernel(GcsGraphView G, GcsStateView St, GcsPerfTables T, Ctrl *ctrl_
     }
     if (threadIdx.x == GCS_COPY_THREAD) gcs_bulk_wait_read();   // shared memory stays valid until the last stores have read it
 #undef STAGE
-    if (INNER) {     // one partial per thread block, summed in a fixed order (static tile assignment: reproducible run to run)
+    if (INNER && !BATCH) {     // one partial per thread block, summed in a fixed order (static tile assignment: reproducible run to run)
 #pragma unroll
         for (int o = 16; o; o >>= 1) rin += __shfl_xor_sync(0xffffffffu, rin, o);
         __syncthreads();                                  // the work arrays are free
@@ -268,7 +269,8 @@ __device__ void control_apply(Ctrl *ctrl, const GcsParams &p, long long n_x, lon
     // abs_stop (the "residual < tol" metric): the inexact x-update's own residual counts too — an iterate whose consensus
     // residuals are small while its vertex programs still violate their cone constraints is not a solution
     const bool ref = p.stop_ref && pri_g >= 0.0 && dual_g >= 0.0;
-    const bool opt = p.abs_stop ? (inner >= 0.0 && fmax(fmax(ref ? pri_g : pri, ref ? dual_g : dual), inner) < p.abs_tol)
+    const double tol = ctrl->abs_tol > 0.0 ? ctrl->abs_tol : p.abs_tol;
+    const bool opt = p.abs_stop ? (inner >= 0.0 && fmax(fmax(ref ? pri_g : pri, ref ? dual_g : dual), inner) < tol)
                                 : (pri < eps_pri && dual < eps_dual);        // :712
     if (opt) { ctrl->opt = 1; ctrl->stop = 1; }
 }
@@ -582,56 +584,77 @@ __global__ void control_kernel(Ctrl *ctrl, GcsParams p, long long n_x, long long
 // ------------------------------------------------------------------------------------------ batched K2-K5
 // Independent problems packed block-diagonally (BASELINE config "batch of 4096 queries"): one block per problem
 // does that problem's edges, its own residual sums and its own rho / stop decision — no communication, and a
-// problem that has converged stops costing anything.
+// problem that has converged stops costing anything.  The per-edge arithmetic is edge_frames_kernel's (the same helpers: local
+// frames and over-relaxation as on one problem; a batch has no edge_counted weights).
+// sums[6]: 0 in the exact mode (pt_res null); in the perf mode -1 until the problem's inner residual is active (Ctrl.inner_active,
+// set by gcsadmm_run), then the sum of its items in pt_res / vt_res, written by K1 of this iteration (a problem's blocks and
+// vertices are contiguous and added in a fixed order: reproducible run to run).  GRES (check variant, local frames): sums[7], [8]
+// in global coordinates for the problems whose inner residual is active; -1 otherwise.
 #define BATCH_THREADS 128
+template <bool OA, bool GRES>
 __global__ void __launch_bounds__(BATCH_THREADS)
-batched_edge_kernel(int nP, const int *__restrict__ prob_eoff, int nHown, const int *__restrict__ edge_he_tail,
-                    const int *__restrict__ edge_he_head, const double *__restrict__ xc, double *__restrict__ mu,
-                    double *__restrict__ z, Ctrl *ctrl_all, GcsParams p, const long long *__restrict__ prob_nx,
-                    const long long *__restrict__ prob_nmu, double *hist, int hist_cap) {
-    __shared__ double sh[BATCH_THREADS / 32][6];
+batched_edge_kernel(int nP, const int *__restrict__ prob_eoff, const int *__restrict__ prob_voff, const int *__restrict__ edge_he_tail,
+                    const int *__restrict__ edge_he_head, const double *__restrict__ edge_delta, const double *__restrict__ edge_cent,
+                    const double *__restrict__ xc, double *__restrict__ mu, double *__restrict__ z, Ctrl *ctrl_all, GcsParams p,
+                    const long long *__restrict__ prob_nx, const long long *__restrict__ prob_nmu, double *hist, int hist_cap,
+                    const int *__restrict__ blk_off, const double *__restrict__ pt_res, const double *__restrict__ vt_res) {
+    __shared__ double sh[BATCH_THREADS / 32][9];
     for (int q = blockIdx.x; q < nP; q += gridDim.x) {
         Ctrl *ctrl = ctrl_all + q;
         if (ctrl->stop && !ctrl->ignore_stop) continue;
-        const double ms = ctrl->mu_scale;
-        double r2 = 0, dz2 = 0, x2 = 0, z2 = 0, m2 = 0, bad = 0;
+        const double ms = ctrl->mu_scale, oa = p.outer_alpha, ob = 1.0 - p.outer_alpha;
+        const bool inner = pt_res && ctrl->inner_active, gres = GRES && inner;
+        double r2 = 0, dz2 = 0, x2 = 0, z2 = 0, m2 = 0, bad = 0, rin = 0, r2g = 0, dz2g = 0;
         for (int e = prob_eoff[q] + threadIdx.x; e < prob_eoff[q + 1]; e += blockDim.x) {
             const int ht = edge_he_tail[e], hh = edge_he_head[e];
-            double xt[5], xh[5], zn[5];
+            double xt[5], xh[5], zo[5], mt[5], mh[5];
 #pragma unroll
-            for (int c = 0; c < 5; ++c) { xt[c] = xc[5 * (size_t)ht + c]; xh[c] = xc[5 * (size_t)hh + c]; }
+            for (int c = 0; c < 5; ++c) { xt[c] = xc[5 * (size_t)ht + c]; xh[c] = xc[5 * (size_t)hh + c]; zo[c] = z[5 * (size_t)e + c]; }
 #pragma unroll
-            for (int c = 0; c < 5; ++c) {
-                const double zo = z[5 * (size_t)e + c];
-                zn[c] = 0.5 * (xt[c] + xh[c]);
-                const double dd = zn[c] - zo;
-                dz2 += dd * dd; z2 += zn[c] * zn[c];
-                z[5 * (size_t)e + c] = zn[c];
-            }
+            for (int c = 0; c < 5; ++c) { mt[c] = mu[5 * (size_t)ht + c]; mh[c] = mu[5 * (size_t)hh + c]; }
+            const double d0 = edge_delta ? edge_delta[2 * (size_t)e] : 0.0, d1 = edge_delta ? edge_delta[2 * (size_t)e + 1] : 0.0;
+            double at[5], ah[5], zn[5], bz[5], dd[5];
+            edge_z_update<OA>(xt, xh, zo, d0, d1, oa, ob, at, ah, zn, bz);
 #pragma unroll
-            for (int c = 0; c < 5; ++c) {
-                const double rt = zn[c] - xt[c], mt = ms * mu[5 * (size_t)ht + c] + rt;
-                mu[5 * (size_t)ht + c] = mt; r2 += rt * rt; x2 += xt[c] * xt[c]; m2 += mt * mt;
-                const double rh = zn[c] - xh[c], mh = ms * mu[5 * (size_t)hh + c] + rh;
-                mu[5 * (size_t)hh + c] = mh; r2 += rh * rh; x2 += xh[c] * xh[c]; m2 += mh * mh;
+            for (int c = 0; c < 5; ++c) { dd[c] = zn[c] - zo[c]; z[5 * (size_t)e + c] = zn[c]; }
+            const double db2 = dd[2] - d0 * dd[4], db3 = dd[3] - d1 * dd[4];
+            dz2 += 0.5 * copies_sq(dd, db2, db3);
+            z2 += 0.5 * copies_sq(zn, bz[2], bz[3]);
+            half_edge_dual(bz, xt, at, mt, ms, mu, 5 * (size_t)ht, true, r2, x2, m2);
+            half_edge_dual(zn, xh, ah, mh, ms, mu, 5 * (size_t)hh, true, r2, x2, m2);
+            if (gres) {      // the expressions of edge_frames_kernel<OA, true>
+                const double cu0 = edge_cent[2 * (size_t)e], cu1 = edge_cent[2 * (size_t)e + 1], cw0 = cu0 - d0, cw1 = cu1 - d1;
+                const double g0 = dd[0] + dd[4] * cu0, g1 = dd[1] + dd[4] * cu1, g2 = dd[2] + dd[4] * cw0, g3 = dd[3] + dd[4] * cw1;
+                dz2g += g0 * g0 + g1 * g1 + g2 * g2 + g3 * g3 + dd[4] * dd[4];
+                double ry = bz[4] - xt[4], a0 = bz[0] - xt[0] + ry * cu0, a1 = bz[1] - xt[1] + ry * cu1, a2 = bz[2] - xt[2] + ry * cu0, a3 = bz[3] - xt[3] + ry * cu1;
+                r2g += a0 * a0 + a1 * a1 + a2 * a2 + a3 * a3 + ry * ry;
+                ry = zn[4] - xh[4]; a0 = zn[0] - xh[0] + ry * cu0; a1 = zn[1] - xh[1] + ry * cu1; a2 = zn[2] - xh[2] + ry * cw0; a3 = zn[3] - xh[3] + ry * cw1;
+                r2g += a0 * a0 + a1 * a1 + a2 * a2 + a3 * a3 + ry * ry;
             }
         }
+        if (inner) {         // the problem's squared inner residual: its half-edge point items, then its path-length items
+            const int va = prob_voff[q], vb = prob_voff[q + 1];
+            for (int j = 2 * blk_off[va] + threadIdx.x; j < 2 * blk_off[vb]; j += blockDim.x) rin += pt_res[j];
+            for (int v = va + threadIdx.x; v < vb; v += blockDim.x) rin += vt_res[v];
+        }
         if (!isfinite(r2) || !isfinite(dz2) || !isfinite(x2) || !isfinite(z2)) bad = 1.0;
-        double vals[6] = {r2, dz2, x2, z2, m2, bad};
+        double vals[9] = {r2, dz2, x2, z2, m2, bad, rin, r2g, dz2g};
 #pragma unroll
-        for (int k = 0; k < 6; ++k)
+        for (int k = 0; k < 9; ++k)
 #pragma unroll
             for (int o = 16; o; o >>= 1) vals[k] += __shfl_xor_sync(0xffffffffu, vals[k], o);
         const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
         if (lane == 0)
-            for (int k = 0; k < 6; ++k) sh[warp][k] = vals[k];
+            for (int k = 0; k < 9; ++k) sh[warp][k] = vals[k];
         __syncthreads();
         if (threadIdx.x == 0) {
-            for (int k = 0; k < 6; ++k) {
+            for (int k = 0; k < 9; ++k) {
                 double sum = 0.0;
                 for (int w2 = 0; w2 < BATCH_THREADS / 32; ++w2) sum += sh[w2][k];
                 ctrl->sums[k] = sum;
             }
+            if (!inner) ctrl->sums[6] = pt_res ? -1.0 : 0.0;      // perf mode: not computed in this iteration | exact mode: 0
+            if (!gres) ctrl->sums[7] = ctrl->sums[8] = -1.0;
             control_apply(ctrl, p, prob_nx[q], prob_nmu[q], hist + (size_t)q * 3 * hist_cap, hist_cap);
         }
         __syncthreads();
@@ -684,10 +707,10 @@ static int reset_ctrl(GcsHandle *h) {
 }
 
 static void free_perf(GcsHandle *h) {
-    void *pp[] = {h->p_vclass, h->p_cone_off, h->p_blk_off, h->p_blk_rec, h->p_vrec, h->p_tile_rec, h->p_cls_tab, h->p_cone, h->p_tstate, h->p_tn, h->p_edge_delta, h->p_edge_cent, h->p_tile_res};
+    void *pp[] = {h->p_vclass, h->p_cone_off, h->p_blk_off, h->p_blk_rec, h->p_vrec, h->p_tile_rec, h->p_cls_tab, h->p_cone, h->p_tstate, h->p_tn, h->p_edge_delta, h->p_edge_cent, h->p_tile_res, h->p_pt_res, h->p_vt_res};
     for (void *q : pp) if (q) cudaFree(q);
     h->p_vclass = h->p_cone_off = h->p_blk_off = h->p_blk_rec = h->p_vrec = h->p_tile_rec = nullptr;
-    h->p_cls_tab = h->p_cone = h->p_tstate = h->p_tn = h->p_edge_delta = h->p_edge_cent = h->p_tile_res = nullptr;
+    h->p_cls_tab = h->p_cone = h->p_tstate = h->p_tn = h->p_edge_delta = h->p_edge_cent = h->p_tile_res = h->p_pt_res = h->p_vt_res = nullptr;
     h->perf_on = 0;
 }
 static void drop_graph(GcsHandle *h) {
@@ -700,7 +723,7 @@ extern "C" int gcsadmm_destroy(GcsHandle *h) {
     cudaSetDevice(h->device);
     void *ptrs[] = {h->poly_off, h->he_off, h->he_edge, h->edge_he_tail, h->edge_he_head, h->polyA, h->polyb, h->cent,
                     h->he_flags, h->vtype, h->edge_counted, h->xc, h->mu, h->z, h->x_v, h->z_v, h->y_v, h->ws, h->partials, h->hist, h->ctrl,
-                    h->vprob, h->prob_eoff, h->prob_nx, h->prob_nmu};
+                    h->vprob, h->prob_voff, h->prob_eoff, h->prob_nx, h->prob_nmu};
     for (void *p : ptrs) if (p) cudaFree(p);
     if (h->ctrl_host) cudaFreeHost(h->ctrl_host);
     free(h->he_prob_host);
@@ -817,6 +840,7 @@ static int create_impl(GcsHandle *h, const GcsGraph *g) {
             nx[q] = 9 * nv + 18 * ne; nm[q] = 10 * ne;
         }
         rc = upload(&h->vprob, vp, (size_t)g->nV);
+        if (!rc) rc = upload(&h->prob_voff, g->prob_voff, (size_t)h->nP + 1);
         if (!rc) rc = upload(&h->prob_eoff, g->prob_eoff, (size_t)h->nP + 1);
         if (!rc) rc = upload(&h->prob_nx, nx, (size_t)h->nP);
         if (!rc) rc = upload(&h->prob_nmu, nm, (size_t)h->nP);
@@ -893,13 +917,17 @@ static int launch_k1(GcsHandle *h) {
 #define INNER_ARGS(h) ((h)->perf_on && (h)->inner_on ? (h)->p_tile_res : nullptr), ((h)->perf_on && (h)->nP == 1 ? ((h)->inner_on ? (h)->perf_grid : -1) : 0)
 // K2-K5.  fuse: the control step runs inside the edge kernel's last block (single GPU); otherwise only sums[] is produced
 static int launch_edge(GcsHandle *h, int fuse) {
+    const bool oa = h->p.outer_alpha != 1.0;
     if (h->nP > 1) {   // edges, sums and control of every problem in one launch
         const int blocks = h->nP < 148 * 16 ? h->nP : 148 * 16;
-        batched_edge_kernel<<<blocks, BATCH_THREADS, 0, h->stream>>>(h->nP, h->prob_eoff, h->nHown, h->edge_he_tail, h->edge_he_head, h->xc, h->mu, h->z,
-                                                                     h->ctrl, h->p, h->prob_nx, h->prob_nmu, h->hist, h->hist_cap);
+        const bool pf = h->perf_on, gres = pf && h->inner_on && h->p_edge_delta && h->p_edge_cent;
+        auto *k = gres ? (oa ? batched_edge_kernel<true, true> : batched_edge_kernel<false, true>)
+                       : (oa ? batched_edge_kernel<true, false> : batched_edge_kernel<false, false>);
+        k<<<blocks, BATCH_THREADS, 0, h->stream>>>(h->nP, h->prob_eoff, h->prob_voff, h->edge_he_tail, h->edge_he_head, pf ? h->p_edge_delta : nullptr,
+            pf ? h->p_edge_cent : nullptr, h->xc, h->mu, h->z, h->ctrl, h->p, h->prob_nx, h->prob_nmu, h->hist, h->hist_cap,
+            pf ? h->p_blk_off : nullptr, pf ? h->p_pt_res : nullptr, pf ? h->p_vt_res : nullptr);
         return 0;
     }
-    const bool oa = h->p.outer_alpha != 1.0;
     if (h->edge_coop && h->nHghost == 0 && !h->edge_counted && !(h->perf_on && h->inner_on)) {     // single-GPU throughput path
         const int nchunks = (h->nE + 31) / 32;
         int blocks = (nchunks + COOP_WARPS - 1) / COOP_WARPS;
@@ -1024,15 +1052,38 @@ extern "C" int gcsadmm_run(GcsHandle *h, int max_iters, GcsStatus *st) {
         CK(cudaGetLastError());
         rc = fetch_ctrl(h); if (rc) return rc;
         done += chunk;
-        if (h->perf_on && h->nP == 1 && h->p.abs_stop) {
+        if (h->perf_on && h->p.abs_stop) {
             // near the absolute target the K1 variant that also measures the inner residual takes over (the stop test needs it);
             // far from it the throughput variant runs.  Every rank of a partitioned run sees the same control block, so all switch together.
-            const int want = fmax(h->ctrl_host->pri, h->ctrl_host->dual) < 4.0 * h->p.abs_tol;
+            // Batch: the same rule per problem, at the same chunk boundaries as its stand-alone run; the INNER variant runs while any
+            // problem that has not stopped needs it (the others' iterates do not depend on which K1 variant runs)
+            int want = 0, changed = 0;
+            for (int q = 0; q < h->nP; ++q) {
+                Ctrl &c = h->ctrl_host[q];
+                const int a = fmax(c.pri, c.dual) < 4.0 * (c.abs_tol > 0.0 ? c.abs_tol : h->p.abs_tol);
+                changed |= a != c.inner_active;
+                c.inner_active = a;
+                want |= a && (h->nP == 1 || !c.stop);
+            }
+            // (the control blocks on the device equal ctrl_host: fetch_ctrl has just synchronised the stream)
+            if (changed && h->nP > 1) CK(cudaMemcpyAsync(h->ctrl, h->ctrl_host, sizeof(Ctrl) * h->nP, cudaMemcpyHostToDevice, h->stream));
             if (want != h->inner_on) { h->inner_on = want; drop_graph(h); }
         }
     }
     if (st) fill_status(h, st);
     if (any_diverged(h)) return set_err(GCS_E_DIVERGED, "non-finite residuals (divergence)%s", "");
+    return 0;
+}
+
+extern "C" int gcsadmm_set_problem_tolerance(GcsHandle *h, const double *abs_tol) {
+    if (!h || !abs_tol) return set_err(GCS_E_INVALID, "null argument%s", "");
+    for (int q = 0; q < h->nP; ++q)
+        if (!isfinite(abs_tol[q]) || abs_tol[q] < 0.0) return set_err(GCS_E_INVALID, "a problem tolerance must be finite and >= 0%s", "");
+    CK(cudaSetDevice(h->device));
+    int rc = fetch_ctrl(h); if (rc) return rc;
+    for (int q = 0; q < h->nP; ++q) h->ctrl_host[q].abs_tol = abs_tol[q];
+    CK(cudaMemcpyAsync(h->ctrl, h->ctrl_host, sizeof(Ctrl) * h->nP, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 
@@ -1361,6 +1412,8 @@ extern "C" int gcsadmm_enable_perf(GcsHandle *h, const GcsPerfConfig *c) {
     if (!rc) rc = upload(&h->p_tstate, (const double *)nullptr, 12 * (size_t)c->n_blocks);
     if (!rc) rc = upload(&h->p_tn, (const double *)nullptr, 2 * (size_t)h->nV);
     if (!rc) rc = upload(&h->p_tile_res, (const double *)nullptr, (size_t)c->n_tiles);
+    if (!rc && h->vprob) rc = upload(&h->p_pt_res, (const double *)nullptr, 2 * (size_t)c->n_blocks);
+    if (!rc && h->vprob) rc = upload(&h->p_vt_res, (const double *)nullptr, (size_t)h->nV);
     if (!rc && c->edge_delta) rc = upload(&h->p_edge_delta, c->edge_delta, 2 * (size_t)h->nE);
     if (!rc && c->edge_delta && c->edge_cent) rc = upload(&h->p_edge_cent, c->edge_cent, 2 * (size_t)h->nE);
     if (rc) { free_perf(h); return rc; }
@@ -1370,6 +1423,7 @@ extern "C" int gcsadmm_enable_perf(GcsHandle *h, const GcsPerfConfig *c) {
     h->PT.blk_off = h->p_blk_off; h->PT.blk_rec = h->p_blk_rec; h->PT.vrec = h->p_vrec; h->PT.tile_rec = h->p_tile_rec;
     h->PT.ntiles = c->n_tiles; h->PT.tstate = h->p_tstate; h->PT.tn = h->p_tn; h->PT.inner_iters = c->inner_iters;
     h->PT.alpha = c->alpha; h->PT.kappa = c->kappa; h->PT.theta = c->theta > 0.0 ? c->theta : 1.0; h->PT.edge_delta = h->p_edge_delta; h->PT.tile_res = h->p_tile_res;
+    h->PT.pt_res = h->p_pt_res; h->PT.vt_res = h->p_vt_res;
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, h->device));
     const size_t bytes = (size_t)(h->PL.work + 2 * h->PL.stage) * sizeof(double);      // work arrays + two stage buffers

@@ -71,6 +71,8 @@ struct GcsPerfTables {
                                // own region (polytopes / cones shifted by cent[v]); the two copies of an edge e = (u, w) then agree through
                                // x_head = z_e,  x_tail = B_e z_e  with  B_e (p1, p2, y) = (p1, p2 - y delta_e, y),  delta_e = cent[u] - cent[w]
     double *tile_res;          // [grid] or null (host emulation); out: squared INNER residual summed over the tiles a thread block walked (INNER kernel variant)
+    double *pt_res, *vt_res;   // batched INNER variant: the same residual per item instead, so that each problem can add up its own share —
+                               // [2 B] one per half-edge point item j = 2 b + i, [nV] one per path-length item
 };
 
 // shared memory of one tile (offsets in doubles).  Two regions: the STAGED arrays that arrive by bulk copies (state t, cone
@@ -336,7 +338,8 @@ GCS_DEV void gcs_tstep(double *t, const double *e, double p0, double p1, double 
 // bar_next): the stores drain during P1 - P2 and the loads land during P3 - P8, without holding the block at a barrier.
 // INNER: also accumulate (into `rin`, per thread) the squared inner residual  |(M u + m0) - c|^2  of the tile's pairs after the
 // last pass — compiled in only for the kernel variant the host switches to near convergence (gcsadmm_run), so the throughput
-// path carries none of it.
+// path carries none of it.  INNER and BATCH: each item's share is stored in T.pt_res / T.vt_res instead, so that the edge kernel can
+// add up every problem's own residual.
 // BATCH: the tile's vertices belong to several problems, each with its own control block ctrl_all[GCS_VI_ACTIVE of the vertex]
 // (rho, mu_scale, stop flag per vertex); otherwise one problem, ctrl_all.
 template <bool INNER, bool BATCH>
@@ -531,8 +534,10 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
             const double *co = cout + GCS_NCX * vl, *tab = T.cls_tab + (size_t)GCS_CLS_STRIDE * w[GCS_VI_CLS], *e = eS + 6 * j;
             const double u0 = gcs_block_u(rS, co, tab, info, b, 2 * i), u1 = gcs_block_u(rS, co, tab, info, b, 2 * i + 1), u4 = gcs_block_u(rS, co, tab, info, b, 4);
             double *t = tS + 6 * j;
-            gcs_tstep<INNER>(t, e, u0, u1, u4, alpha, last, rin);                                     // fam 0: (a_i, y_e)
-            if (!((info >> 10) & 1)) gcs_tstep<INNER>(t + 3, e + 3, co[2 * i] - u0, co[2 * i + 1] - u1, 1.0 - u4, alpha, last, rin);   // fam 1: (x_i - a_i, 1 - y_e)
+            double ri = 0.0, &ra = INNER && BATCH ? ri : rin;           // batched: the item's own share, stored below
+            gcs_tstep<INNER>(t, e, u0, u1, u4, alpha, last, ra);                                      // fam 0: (a_i, y_e)
+            if (!((info >> 10) & 1)) gcs_tstep<INNER>(t + 3, e + 3, co[2 * i] - u0, co[2 * i + 1] - u1, 1.0 - u4, alpha, last, ra);    // fam 1: (x_i - a_i, 1 - y_e)
+            if (INNER && BATCH && last) T.pt_res[2 * (size_t)b0 + j] = ri;
             const int h = bhe(b);
             if (last && h >= 0) {
                 // out-edge: point i is slots 2 i, 2 i + 1 (own first point | other's first point == own second point, C5);
@@ -557,7 +562,8 @@ GCS_DEV void gcs_perf_tile(const GcsGraphView &G, const GcsStateView &St, const 
                 const double *zz = cout + GCS_NCX * i + 4;
                 if (INNER && last) {
                     const double ic = 1.0 / (2.0 - alpha), r0 = (zz[0] - zz[2]) - ic * (tnS[2 * i] + enS[2 * i]), r1 = (zz[1] - zz[3]) - ic * (tnS[2 * i + 1] + enS[2 * i + 1]);
-                    rin += r0 * r0 + r1 * r1;
+                    if (BATCH) T.vt_res[v0 + i] = r0 * r0 + r1 * r1;
+                    else rin += r0 * r0 + r1 * r1;
                 }
                 tnS[2 * i] = alpha * (zz[0] - zz[2]) + enS[2 * i]; tnS[2 * i + 1] = alpha * (zz[1] - zz[3]) + enS[2 * i + 1];
             }

@@ -22,6 +22,7 @@ EXPORTS = [
     "gcsadmm_get_state", "gcsadmm_set_state", "gcsadmm_time_steps", "gcsadmm_time_window", "gcsadmm_solve_host",
     "gcsadmm_scratch_bytes", "gcsadmm_flush_l2", "gcsadmm_get_problem_status", "gcsadmm_get_problem_history", "gcsadmm_enable_perf",
     "gcsadmm_get_perf_state", "gcsadmm_set_perf_state", "gcsadmm_peer_export", "gcsadmm_peer_connect", "gcsadmm_peer_error",
+    "gcsadmm_set_problem_tolerance",
 ]
 
 
@@ -87,6 +88,7 @@ def load():
     L.gcsadmm_step.argtypes = [C.c_void_p, C.c_int]
     L.gcsadmm_get_status.argtypes = [C.c_void_p, C.POINTER(GcsStatus)]
     L.gcsadmm_get_problem_status.argtypes = [C.c_void_p, C.c_int, C.POINTER(GcsStatus)]
+    L.gcsadmm_set_problem_tolerance.argtypes = [C.c_void_p, C.c_void_p]
     L.gcsadmm_get_problem_history.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
     for f in ("gcsadmm_vertex_update", "gcsadmm_edge_update", "gcsadmm_control"):
         getattr(L, f).argtypes = [C.c_void_p]
@@ -268,6 +270,13 @@ class Solver:
         st = GcsStatus()
         _check(load().gcsadmm_get_problem_status(self._h, int(p), C.byref(st)))
         return st.as_dict()
+
+    def set_problem_tolerance(self, tols):
+        """each problem's own ``abs_tol`` of the absolute stop rule (one value per packed problem; 0: the handle's ``abs_tol``)"""
+        t = np.ascontiguousarray(tols, np.float64).reshape(-1)
+        if t.shape[0] != self._gs.nP:
+            raise ValueError(f"{self._gs.nP} tolerances expected, got {t.shape[0]}")
+        _check(load().gcsadmm_set_problem_tolerance(self._h, _ptr(t)))
 
     def problem_history(self, p):
         cap = self.params.max_it + 2

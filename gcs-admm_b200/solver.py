@@ -13,10 +13,10 @@ import time
 import numpy as np
 
 from . import lib
-from .graph import build_graph, pack_graph
+from .graph import build_graph, pack_batch, pack_graph
 from .rounding import compute_cost, rounding
 
-__all__ = ["solve", "MAX_IT"]
+__all__ = ["solve", "solve_batch", "MAX_IT"]
 
 MAX_IT = 1000     # reference admm_solver_v3.py:651
 
@@ -73,15 +73,9 @@ def solve(As, bs, n, *, device=0, max_it=MAX_IT, round_solution=True, seed=None,
     else:
         V, E, I_v_in, I_v_out, g = graph
     t0 = time.perf_counter()
-    if mode not in ("parity", "perf"):
-        raise ValueError("mode must be 'parity' or 'perf'")
+    max_it = _mode_defaults(mode, max_it, params)
     if mode == "perf":
-        if max_it == MAX_IT:
-            max_it = PERF_MAX_IT
-        params.setdefault("abs_stop", 1)
         params.setdefault("abs_tol", perf_abs_tol(g))
-        params.setdefault("frac", PERF_ADAPT_WINDOW / max_it)
-        params.setdefault("check_every", 64)
     if one_call and mode == "parity":
         out = lib.solve_host(g, device=device, max_iters=max_it, max_it=max_it, **params)
     else:
@@ -99,6 +93,65 @@ def solve(As, bs, n, *, device=0, max_it=MAX_IT, round_solution=True, seed=None,
     st = out["status"]
     if verbose:
         print(f"it = {st['iterations']}/{max_it}, pri_res_seq[-1]={st['pri_res']}, dual_res_seq[-1]={st['dual_res']}")
+    return _result(out, V, E, I_v_out, As, bs, n, mode, solve_time, round_solution, seed, rounding_kw)
+
+
+def solve_batch(queries, *, device=0, max_it=MAX_IT, round_solution=True, seed=None, mode="parity", inner_iters=1,
+                rounding_kw=None, frames="global", warm_start=None, **params):
+    """Solve many independent problems (start / goal queries) in one handle: ``queries`` is a list of ``(As, bs)`` in the
+    reference's format (n = 2).  The problems are packed block-diagonally (``graph.pack_batch``); each keeps its own residuals,
+    rho, stop decision and, in the perf mode, its own tolerance ``perf_abs_tol`` (unless ``abs_tol`` is given).  A query's
+    iterates, iteration count and stop are those of ``solve()`` on it alone with the same options.
+
+    Takes ``solve()``'s keyword arguments and returns a list with one ``solve()`` result dict per query; ``solve_time`` is the
+    time of the whole batch.  Rounding runs per query on the host."""
+    built = []
+    for As, bs in queries:
+        V, E, I_v_in, I_v_out = build_graph(As, bs)
+        built.append((V, E, I_v_out, pack_graph(As, bs, V, E)))
+    big = pack_batch([b[3] for b in built])
+    t0 = time.perf_counter()
+    max_it = _mode_defaults(mode, max_it, params)
+    tols = [perf_abs_tol(b[3]) for b in built] if mode == "perf" and "abs_tol" not in params else None
+    s = lib.Solver(big, device=device, max_it=max_it, **params)
+    try:
+        if mode == "perf":
+            s.enable_perf(inner_iters=inner_iters, frames=frames)
+            if tols is not None:
+                s.set_problem_tolerance(tols)
+            if warm_start:
+                s.warm_start(field=warm_start)
+        s.run(max_it)
+        x_v, z_v, y_v, z_e = s.solution()
+        per = [(s.problem_status(q), s.problem_history(q)) for q in range(len(built))]
+    finally:
+        s.close()
+    solve_time = time.perf_counter() - t0
+    out = []
+    for q, ((V, E, I_v_out, g), (st, (rho, pri, dual))) in enumerate(zip(built, per)):
+        v0, v1, e0, e1 = big.prob_voff[q], big.prob_voff[q + 1], big.prob_eoff[q], big.prob_eoff[q + 1]
+        arrays = dict(status=st, x_v=x_v[v0:v1], z_v=z_v[v0:v1], y_v=y_v[v0:v1], z_e=z_e[e0:e1], rho_seq=rho, pri_res_seq=pri, dual_res_seq=dual)
+        As, bs = queries[q]
+        out.append(_result(arrays, V, E, I_v_out, As, bs, 2, mode, solve_time, round_solution, seed, rounding_kw))
+    return out
+
+
+def _mode_defaults(mode, max_it, params):
+    """the perf mode's stop rule and adaptation window (DESIGN.md section 5a) unless the caller set them -> max_it"""
+    if mode not in ("parity", "perf"):
+        raise ValueError("mode must be 'parity' or 'perf'")
+    if mode == "perf":
+        if max_it == MAX_IT:
+            max_it = PERF_MAX_IT
+        params.setdefault("abs_stop", 1)
+        params.setdefault("frac", PERF_ADAPT_WINDOW / max_it)
+        params.setdefault("check_every", 64)
+    return max_it
+
+
+def _result(out, V, E, I_v_out, As, bs, n, mode, solve_time, round_solution, seed, rounding_kw):
+    """one problem's arrays (status, x_v, z_v, y_v, z_e, rho / pri / dual sequences) -> the result dict of ``solve()``"""
+    st = out["status"]
     x_v_sol = {v: out["x_v"][i].copy() for i, v in enumerate(V)}        # :745
     y_v_sol = {v: float(out["y_v"][i]) for i, v in enumerate(V)}        # :746
     y_e_sol = {e: float(out["z_e"][i, 4]) for i, e in enumerate(E)}     # :747

@@ -42,14 +42,19 @@ def cost_to_go(g, field="dijkstra", return_next=False):
     """(J[nE], grad[nE, 2]): cost-to-go from the portal of every edge and its gradient (minus the unit direction of travel).
     ``field="euclid"``: straight-line distance to the target (exact on obstacle-free maps); ``"dijkstra"``: shortest path over
     the portal graph (portal of e = (u, w) -> portal of f = (w, x), weight = their distance), valid for any region graph.
-    Edges that cannot reach the target get J = 0, grad = 0 (their flow is forced to zero by the presolve anyway)."""
+    Edges that cannot reach the target get J = 0, grad = 0 (their flow is forced to zero by the presolve anyway).
+    A block-diagonal batch (``graph.pack_batch``) has one target per problem (``g.dsts``): every edge is measured to its own
+    problem's target, and since the problems are disconnected one search gives each of them its own field."""
     p = portal_points(g)
     c = np.asarray(g.interior_points())
-    tgt = c[g.dst]
     nE = g.nE
+    dsts = np.atleast_1d(np.asarray(getattr(g, "dsts", [g.dst]), np.int64))
+    eoff = getattr(g, "prob_eoff", None)
+    prob = np.searchsorted(np.asarray(eoff), np.arange(nE), side="right") - 1 if eoff is not None else np.zeros(nE, np.int64)
+    tgt = c[dsts[prob]]                                  # [nE, 2]: the target of every edge's problem
     tail, head = np.asarray(g.edge_tail, np.int64), np.asarray(g.edge_head, np.int64)
     if field == "euclid":
-        d = tgt[None, :] - p
+        d = tgt - p
         J = np.linalg.norm(d, axis=1)
         grad = -d / np.where(J > 0, J, 1.0)[:, None]
         if return_next:
@@ -72,18 +77,18 @@ def cost_to_go(g, field="dijkstra", return_next=False):
     keep = tail[ei] != head[fo]                          # no immediate U-turn
     ei, fo = ei[keep], fo[keep]
     w = np.linalg.norm(p[fo] - p[ei], axis=1) + 1e-12
-    # node nE = the target: every edge into t connects to it at the remaining distance
-    into_t = np.nonzero(head == g.dst)[0]
+    # node nE = the target(s): every edge into t connects to it at the remaining distance
+    into_t = np.nonzero(np.isin(head, dsts[dsts >= 0]))[0]
     rows = np.concatenate([fo, np.full(into_t.shape[0], nE)])          # reversed arcs: search from the target
     cols = np.concatenate([ei, into_t])
-    vals = np.concatenate([w, np.linalg.norm(tgt[None, :] - p[into_t], axis=1) + 1e-12])
+    vals = np.concatenate([w, np.linalg.norm(tgt[into_t] - p[into_t], axis=1) + 1e-12])
     A = csr_matrix((vals, (rows, cols)), shape=(nE + 1, nE + 1))
     dist, pred = dijkstra(A, directed=True, indices=nE, return_predecessors=True)
     J = dist[:nE].copy()
     nxt = pred[:nE]                                      # next portal on the way to the target (nE = the target itself)
     ok = np.isfinite(J) & (nxt >= 0)
     J[~ok] = 0.0
-    to = np.where(nxt[:, None] == nE, tgt[None, :], p[np.clip(nxt, 0, nE - 1)])
+    to = np.where(nxt[:, None] == nE, tgt, p[np.clip(nxt, 0, nE - 1)])
     d = to - p
     n = np.linalg.norm(d, axis=1)
     grad = np.where((ok & (n > 1e-9))[:, None], -d / np.where(n > 1e-9, n, 1.0)[:, None], 0.0)

@@ -134,6 +134,10 @@ int gcsadmm_run(GcsHandle *h, int max_iters, GcsStatus *st);   /* until the stop
 int gcsadmm_step(GcsHandle *h, int k);                         /* exactly k passes, stop rule evaluated but ignored */
 int gcsadmm_get_status(GcsHandle *h, GcsStatus *st);            /* batched handle: worst residuals, max iterations, all-converged */
 int gcsadmm_get_problem_status(GcsHandle *h, int problem, GcsStatus *st);
+/* abs_tol[nP]: each problem's own tolerance of the absolute stop rule (abs_stop), and of the switch to the K1 variant that
+ * measures the inner residual (4 x the tolerance); 0 = GcsParams.abs_tol.  GCS_E_INVALID for a NULL pointer or a negative or
+ * non-finite value */
+int gcsadmm_set_problem_tolerance(GcsHandle *h, const double *abs_tol);
 
 /* the individual kernels (per-kernel parity tests, multi-GPU driver) */
 int gcsadmm_vertex_update(GcsHandle *h);                       /* K1 */
